@@ -4,6 +4,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo (CUDA)
     python bench.py --impl reference --gpus N ...            # CPU arm (no CUDA library loaded)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's calls as DIR/*.npy
 
 Workload = BASELINE.json configs[1]: 10 M synthetic 2x150 bp read pairs, 50 %
 sampled from the genome the table was built from ("human-derived"), --conf 0.5,
@@ -70,7 +71,15 @@ def parse_args():
                     "comma separated; the best one is reported, all are listed")
     ap.add_argument("--no-workloads", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the calls and keep mask of the last timed step to DIR/*.npy "
+                         "(a fixed sample if they exceed 64 MB), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA path only")
+    return args
 
 
 def workload_config(args):
@@ -235,6 +244,25 @@ def workload_offsets(shape, total_bases, seed):
     return off
 
 
+DUMP_BYTES = 64_000_000
+DUMP_SAMPLE = 1 << 21
+DUMP_SEED = 20240601
+
+
+def dump_outputs(out_dir, call, keep):
+    """Writes one step's results (the launches' outputs concatenated in batch order) as call.npy (external taxid,
+    float64: exact for every 32-bit id) and keep.npy (0/1, float32).  Above DUMP_BYTES only a fixed seeded sample
+    of positions is written, with those positions in index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(call)
+    if n * 12 > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(n, DUMP_SAMPLE), replace=False))
+        call, keep = call[idx], keep[idx]
+        np.save(os.path.join(out_dir, "index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "call.npy"), call.astype(np.uint32).astype(np.float64))
+    np.save(os.path.join(out_dir, "keep.npy"), keep.astype(np.float32))
+
+
 # ---------------------------------------------------------------------------------------------
 # CPU side (oracle): the only functions that touch oracle/
 
@@ -373,13 +401,16 @@ def main():
 
     # ---------------- device-resident timing (`value`) ----------------
     sess = Session(db, confidence=CONF, paired=True, max_batch_bases=total + 4096, max_batch_seqs=n_seqs)
-    d_call = torch.empty(n_pairs, dtype=torch.int32, device="cuda")
-    d_keep = torch.empty(n_pairs, dtype=torch.uint8, device="cuda")
+    # one output pair per batch: after the timed loop they hold what the last step computed
+    d_calls = [torch.empty(n_pairs, dtype=torch.int32, device="cuda") for _ in range(n_launch)]
+    d_keeps = [torch.empty(n_pairs, dtype=torch.uint8, device="cuda") for _ in range(n_launch)]
+    d_call, d_keep = d_calls[0], d_keeps[0]
     ext = torch.cuda.ExternalStream(sess.stream)
 
     def launch(i):
-        sess.classify_device(bufs[i % n_launch].data_ptr(), d_off.data_ptr(), n_seqs, total, d_call.data_ptr(),
-                             d_keep.data_ptr())
+        b = i % n_launch
+        sess.classify_device(bufs[b].data_ptr(), d_off.data_ptr(), n_seqs, total, d_calls[b].data_ptr(),
+                             d_keeps[b].data_ptr())
         return sess.sync()
 
     sampler = ClockSampler(dev)
@@ -425,6 +456,8 @@ def main():
         stage[kname] /= n_timed
     lk_per_launch = lookups / n_timed
     sec_per_launch = sectors / n_timed
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, torch.cat(d_calls).cpu().numpy(), torch.cat(d_keeps).cpu().numpy())
 
     # ---------------- e2e through the C ABI with host buffers ----------------
     e2e = None

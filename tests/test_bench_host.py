@@ -6,6 +6,7 @@ import subprocess
 import sys
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -38,6 +39,41 @@ print(json.dumps({"torch": "torch" in sys.modules, "gpu_lib": "libnohuman_gpu" i
     finally:
         sys.argv = saved
     assert ours == line["config"]  # the driver's same_config check
+
+
+def test_dump_outputs_is_bounded_and_repeatable(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    rng = np.random.default_rng(3)
+    small = rng.choice(np.array([0, 9606, 9100404], np.int32), size=1000)
+    bench.dump_outputs(str(tmp_path / "s"), small, (small == 0).astype(np.uint8))
+    assert sorted(os.listdir(tmp_path / "s")) == ["call.npy", "keep.npy"]
+    call = np.load(tmp_path / "s" / "call.npy")
+    assert call.dtype == np.float64 and np.array_equal(call, small)
+    assert np.load(tmp_path / "s" / "keep.npy").dtype == np.float32
+    big = rng.integers(0, 1 << 31, size=10_000_000, dtype=np.int64).astype(np.int32)  # one default step: 10 x 1M pairs
+    keep = (big & 1).astype(np.uint8)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), big, keep)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["call.npy", "index.npy", "keep.npy"]
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64_000_000
+    for f in files:
+        assert np.array_equal(np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f))
+    idx = np.load(tmp_path / "a" / "index.npy").astype(np.int64)
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "call.npy"), big[idx].astype(np.uint32))
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "keep.npy"), keep[idx])
+
+
+def test_steps_must_be_positive(monkeypatch):
+    sys.path.insert(0, ROOT)
+    import bench
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "0"])
+    with pytest.raises(SystemExit):
+        bench.parse_args()
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "3", "--dump-outputs", "d"])
+    args = bench.parse_args()
+    assert args.steps == 3 and args.dump_outputs == "d"
 
 
 def test_workload_shapes():
