@@ -18,6 +18,7 @@
 #include <atomic>
 #include <condition_variable>
 #include <functional>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -101,14 +102,29 @@ int nh_resolve_db_dir(const char *db_dir, std::string &out) {
                       db_dir, db_dir);
 }
 
-static int parse_opts_taxo(nh_db *db, const void *opts, size_t opts_len, const void *taxo,
-                           size_t taxo_len) {
+/* A handle under construction: every failure path releases it through nh_db_close. */
+struct DbCloser {
+  void operator()(nh_db *db) const { nh_db_close(db); }
+};
+using DbPtr = std::unique_ptr<nh_db, DbCloser>;
+
+/* the cell array padded to whole 128-byte lines (zero cells), so a 4-sector group load stays inside the allocation */
+static size_t table_bytes(uint64_t capacity) { return ((capacity + 31) / 32) * 128; }
+
+/* A new handle for `device` with everything it keeps on the host, from the opts.k2d and taxo.k2d images and the
+ * hash.k2d header {capacity, size, key_bits, value_bits}: info, the taxonomy, and every field of params except the
+ * device pointers finish_db sets.  It checks all it reads and makes no CUDA call, so malformed input is reported as
+ * such before any device work, on a machine without a GPU too. */
+static int parse_db(const void *opts, size_t opts_len, const void *taxo, size_t taxo_len, const uint64_t hdr[4],
+                    int device, DbPtr &db) {
+  db.reset(new nh_db());
+  nh_db_info_t &I = db->info;
+  I.device = device;
   /* opts.k2d: raw IndexOptions, up to 64 bytes; older DBs are shorter */
   uint8_t ob[64];
   memset(ob, 0, sizeof ob);
   if (opts_len < 32) return nh_set_error(NH_ERR_IO, "opts.k2d too short (%zu bytes)", opts_len);
   memcpy(ob, opts, opts_len < 64 ? opts_len : 64);
-  nh_db_info_t &I = db->info;
   memcpy(&I.k, ob + 0, 8);
   memcpy(&I.l, ob + 8, 8);
   memcpy(&I.spaced_seed_mask, ob + 16, 8);
@@ -130,7 +146,6 @@ static int parse_opts_taxo(nh_db *db, const void *opts, size_t opts_len, const v
   I.node_count = node_count;
   db->h_parent.resize(node_count);
   db->h_ext.resize(node_count);
-  db->h_ext64.resize(node_count);
   db->h_name.assign(node_count, std::string());
   db->h_rank.assign(node_count, std::string());
   const uint64_t names_at = 32 + node_count * 56, ranks_at = names_at + name_len;
@@ -148,7 +163,6 @@ static int parse_opts_taxo(nh_db *db, const void *opts, size_t opts_len, const v
                           (unsigned long long)ext);
     db->h_parent[i] = (uint32_t)parent;
     db->h_ext[i] = (uint32_t)ext;
-    db->h_ext64[i] = ext;
     if (have_strings && i > 0) {
       uint64_t no, ro;
       memcpy(&no, tb + 32 + i * 56 + 24, 8);
@@ -158,11 +172,7 @@ static int parse_opts_taxo(nh_db *db, const void *opts, size_t opts_len, const v
     }
   }
   db->h_parent[0] = 0;
-  return NH_OK;
-}
-
-static int finish_db(nh_db *db, const uint64_t hdr[4], bool cells_ready = true) {
-  nh_db_info_t &I = db->info;
+  /* hash.k2d header */
   I.capacity = hdr[0];
   I.size = hdr[1];
   I.key_bits = hdr[2];
@@ -182,8 +192,6 @@ static int finish_db(nh_db *db, const uint64_t hdr[4], bool cells_ready = true) 
   if (I.node_count > (1ULL << I.value_bits))
     return nh_set_error(NH_ERR_IO, "taxonomy has more nodes than value_bits can address");
   NhDbParams &P = db->params;
-  memset(&P, 0, sizeof P);
-  P.cells = db->d_cells;
   P.capacity = I.capacity;
   nh_divisor dv = nh_make_divisor(I.capacity);
   P.mod_m = dv.m;
@@ -203,21 +211,34 @@ static int finish_db(nh_db *db, const uint64_t hdr[4], bool cells_ready = true) 
   P.toggle = I.toggle_mask & lmer_mask;
   P.min_hash = I.minimum_acceptable_hash_value;
   P.node_count = (uint32_t)I.node_count;
-  CUDA_TRY(cudaMalloc(&db->d_parent, I.node_count * 4));
-  CUDA_TRY(cudaMalloc(&db->d_ext, I.node_count * 4));
-  CUDA_TRY(cudaMemcpy(db->d_parent, db->h_parent.data(), I.node_count * 4, cudaMemcpyHostToDevice));
-  CUDA_TRY(cudaMemcpy(db->d_ext, db->h_ext.data(), I.node_count * 4, cudaMemcpyHostToDevice));
-  P.parent = db->d_parent;
-  P.ext_id = db->d_ext;
   /* a read can hit at most node_count distinct taxa; k_score_big's shared table holds 16K of them */
   if (I.node_count >= NH_BIG_HASH_SLOTS * 3 / 4) {
     uint32_t slots = 1;
     while (slots < 2 * I.node_count) slots <<= 1;
-    CUDA_TRY(cudaMalloc(&db->d_huge, ((size_t)2 * slots + 4) * 4));
-    CUDA_TRY(cudaMemset(db->d_huge, 0, ((size_t)2 * slots + 4) * 4));
     P.huge_slots = slots;
-    P.huge_table = db->d_huge;
   }
+  return NH_OK;
+}
+
+/* The device side of a handle whose host side is filled in and whose cell array is on its device: the taxonomy
+ * arrays, the huge taxon table, the kernels' set-up, and the miss filter once the cells hold the table. */
+static int finish_db(nh_db *db, bool cells_ready = true) {
+  const size_t taxo_bytes = db->info.node_count * 4;
+  NhDbParams &P = db->params;
+  CUDA_TRY(cudaSetDevice(db->info.device));
+  CUDA_TRY(cudaMalloc(&db->d_parent, taxo_bytes));
+  CUDA_TRY(cudaMalloc(&db->d_ext, taxo_bytes));
+  CUDA_TRY(cudaMemcpy(db->d_parent, db->h_parent.data(), taxo_bytes, cudaMemcpyHostToDevice));
+  CUDA_TRY(cudaMemcpy(db->d_ext, db->h_ext.data(), taxo_bytes, cudaMemcpyHostToDevice));
+  if (P.huge_slots) {
+    const size_t huge_bytes = ((size_t)2 * P.huge_slots + 4) * 4;
+    CUDA_TRY(cudaMalloc(&db->d_huge, huge_bytes));
+    CUDA_TRY(cudaMemset(db->d_huge, 0, huge_bytes));
+  }
+  P.cells = db->d_cells;
+  P.parent = db->d_parent;
+  P.ext_id = db->d_ext;
+  P.huge_table = db->d_huge;
   cudaDeviceProp prop;
   CUDA_TRY(cudaGetDeviceProperties(&prop, db->info.device));
   db->sm_count = prop.multiProcessorCount;
@@ -264,218 +285,163 @@ static int select_device(int device) {
   return NH_OK;
 }
 
+/* db's cell array on the current device: table_bytes(capacity), zeroed */
+static int alloc_cells(nh_db *db) {
+  const size_t bytes = table_bytes(db->info.capacity);
+  const cudaError_t e = cudaMalloc(&db->d_cells, bytes);
+  if (e != cudaSuccess) {
+    db->d_cells = nullptr;
+    cudaGetLastError();
+    return nh_set_error(NH_ERR_NOMEM, "cudaMalloc(%zu) for the hash table on device %d failed: %s", bytes,
+                        db->info.device, cudaGetErrorString(e));
+  }
+  db->owns_cells = true;
+  CUDA_TRY(cudaMemset(db->d_cells, 0, bytes));
+  return NH_OK;
+}
+
+/* The cells of hash.k2d (f is positioned after the header) into db->d_cells, streamed through two pinned staging
+ * buffers so that the multi-GB table never needs a second host copy: reading one chunk overlaps copying the other. */
+static int upload_cells(FILE *f, nh_db *db) {
+  const size_t CH = 64u << 20, total = db->info.capacity * 4;
+  uint8_t *stage[2] = {nullptr, nullptr};
+  cudaEvent_t ev[2] = {nullptr, nullptr};
+  cudaStream_t cs = nullptr;
+  int rc = NH_OK;
+  cudaError_t e = cudaStreamCreate(&cs);
+  for (int i = 0; i < 2 && e == cudaSuccess; i++) e = cudaEventCreate(&ev[i]);
+  for (int i = 0; i < 2 && e == cudaSuccess && rc == NH_OK; i++)
+    if (cudaHostAlloc(&stage[i], CH, cudaHostAllocDefault) != cudaSuccess) {
+      stage[i] = nullptr;
+      cudaGetLastError();
+      rc = nh_set_error(NH_ERR_NOMEM, "pinned staging allocation failed");
+    }
+  size_t done = 0;
+  for (int slot = 0; e == cudaSuccess && rc == NH_OK && done < total; slot ^= 1) {
+    const size_t n = total - done < CH ? total - done : CH;
+    if ((e = cudaEventSynchronize(ev[slot])) != cudaSuccess) break; /* the copy out of this buffer has finished */
+    if (fread(stage[slot], 1, n, f) != n) {
+      rc = nh_set_error(NH_ERR_IO, "hash.k2d: short read");
+      break;
+    }
+    if ((e = cudaMemcpyAsync((uint8_t *)db->d_cells + done, stage[slot], n, cudaMemcpyHostToDevice, cs)) != cudaSuccess ||
+        (e = cudaEventRecord(ev[slot], cs)) != cudaSuccess)
+      break;
+    done += n;
+  }
+  if (cs) {
+    const cudaError_t se = cudaStreamSynchronize(cs); /* no copy may still read a staging buffer when it is freed */
+    if (e == cudaSuccess) e = se;
+  }
+  for (int i = 0; i < 2; i++) {
+    if (stage[i]) cudaFreeHost(stage[i]);
+    if (ev[i]) cudaEventDestroy(ev[i]);
+  }
+  if (cs) cudaStreamDestroy(cs);
+  if (rc == NH_OK && e != cudaSuccess) rc = nh_set_error(NH_ERR_CUDA, "table upload failed: %s", cudaGetErrorString(e));
+  return rc;
+}
+
 extern "C" int nh_db_open_memory(const void *opts, size_t opts_len, const void *taxo, size_t taxo_len,
                                  const uint64_t hash_header[4], const uint32_t *cells,
                                  int cells_on_device, int device, nh_db **out) {
   if (!opts || !taxo || !hash_header || !cells || !out) return nh_set_error(NH_ERR_INVALID, "null argument");
-  int rc = select_device(device);
+  DbPtr db;
+  int rc = parse_db(opts, opts_len, taxo, taxo_len, hash_header, device, db);
+  if (!rc) rc = select_device(device);
   if (rc) return rc;
-  nh_db *db = new nh_db();
-  db->info.device = device;
-  rc = parse_opts_taxo(db, opts, opts_len, taxo, taxo_len);
-  if (rc) {
-    delete db;
-    return rc;
-  }
-  const uint64_t cap = hash_header[0];
   if (cells_on_device) {
-    if (((uintptr_t)cells & 127u) != 0) {
-      delete db;
-      return nh_set_error(NH_ERR_INVALID, "device cell array must be 128-byte aligned");
-    }
-    db->d_cells = const_cast<uint32_t *>(cells);
-    db->owns_cells = false;
+    if (((uintptr_t)cells & 127u) != 0) return nh_set_error(NH_ERR_INVALID, "device cell array must be 128-byte aligned");
+    db->d_cells = const_cast<uint32_t *>(cells); /* adopted: the caller keeps ownership */
   } else {
-    /* padded to whole 128-byte lines (zero cells) so a 4-sector group load stays inside the allocation */
-    const size_t bytes = ((cap + 31) / 32) * 128;
-    cudaError_t e = cudaMalloc(&db->d_cells, bytes);
-    if (e != cudaSuccess) {
-      delete db;
-      return nh_set_error(NH_ERR_NOMEM, "cudaMalloc(%zu) for the hash table failed: %s", bytes,
-                          cudaGetErrorString(e));
-    }
-    db->owns_cells = true;
-    cudaMemset(db->d_cells, 0, bytes);
-    e = cudaMemcpy(db->d_cells, cells, cap * 4, cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) {
-      nh_db_close(db);
-      return nh_set_error(NH_ERR_CUDA, "copying the hash table to the device failed: %s",
-                          cudaGetErrorString(e));
-    }
+    if ((rc = alloc_cells(db.get()))) return rc;
+    const cudaError_t e = cudaMemcpy(db->d_cells, cells, db->info.capacity * 4, cudaMemcpyHostToDevice);
+    if (e != cudaSuccess)
+      return nh_set_error(NH_ERR_CUDA, "copying the hash table to the device failed: %s", cudaGetErrorString(e));
   }
-  rc = finish_db(db, hash_header);
-  if (rc) {
-    nh_db_close(db);
-    return rc;
-  }
-  *out = db;
+  if ((rc = finish_db(db.get()))) return rc;
+  *out = db.release();
   return NH_OK;
 }
 
-/* Zeroed table of `capacity` cells for the synthetic builder (nh_synth.cu);
- * value_bits as build_db.cc picks it: the smallest b with 2^b >= node_count. */
+/* value_bits as build_db.cc picks it: the smallest b with 2^b >= node_count, read here from taxo.k2d's header,
+ * which parse_db then checks with the rest of the image */
 int nh_db_create_empty(const void *opts, size_t opts_len, const void *taxo, size_t taxo_len,
                        uint64_t capacity, int device, nh_db **out) {
-  int rc = select_device(device);
-  if (rc) return rc;
-  nh_db *db = new nh_db();
-  db->info.device = device;
-  rc = parse_opts_taxo(db, opts, opts_len, taxo, taxo_len);
-  if (rc) {
-    delete db;
-    return rc;
-  }
-  uint64_t vb = 1;
-  while ((1ULL << vb) < db->info.node_count) vb++;
-  const size_t bytes = ((capacity + 31) / 32) * 128;
-  cudaError_t e = cudaMalloc(&db->d_cells, bytes);
-  if (e != cudaSuccess) {
-    delete db;
-    return nh_set_error(NH_ERR_NOMEM, "cudaMalloc(%zu) for the hash table failed: %s", bytes,
-                        cudaGetErrorString(e));
-  }
-  db->owns_cells = true;
-  cudaMemset(db->d_cells, 0, bytes);
+  uint64_t node_count = 0, vb = 1;
+  if (taxo_len >= 16) memcpy(&node_count, (const uint8_t *)taxo + 8, 8);
+  while (vb < 31 && (1ULL << vb) < node_count) vb++;
   const uint64_t hdr[4] = {capacity, 0, 32 - vb, vb};
-  rc = finish_db(db, hdr, false); /* the builder fills the cells and calls nh_db_build_filter when it is done */
-  if (rc) {
-    nh_db_close(db);
-    return rc;
-  }
-  *out = db;
+  DbPtr db;
+  int rc = parse_db(opts, opts_len, taxo, taxo_len, hdr, device, db);
+  if (!rc) rc = select_device(device);
+  if (!rc) rc = alloc_cells(db.get());
+  if (!rc) rc = finish_db(db.get(), false);
+  if (rc) return rc;
+  *out = db.release();
   return NH_OK;
 }
 
 extern "C" int nh_db_open(const char *db_dir, int device, nh_db **out) {
   if (!db_dir || !out) return nh_set_error(NH_ERR_INVALID, "null argument");
   std::string dir;
-  int rc = nh_resolve_db_dir(db_dir, dir);
-  if (rc) return rc;
-  rc = select_device(device);
-  if (rc) return rc;
   std::vector<uint8_t> opts, taxo;
-  rc = read_file(dir + "/opts.k2d", opts, 64);
+  int rc = nh_resolve_db_dir(db_dir, dir);
+  if (!rc) rc = read_file(dir + "/opts.k2d", opts, 64);
+  if (!rc) rc = read_file(dir + "/taxo.k2d", taxo, (size_t)-1);
   if (rc) return rc;
-  rc = read_file(dir + "/taxo.k2d", taxo, (size_t)-1);
-  if (rc) return rc;
-  /* hash.k2d: 32-byte header, then capacity x u32; streamed through a pinned
-   * staging buffer so that the multi-GB table never needs a second host copy */
-  std::string hp = dir + "/hash.k2d";
-  FILE *f = fopen(hp.c_str(), "rb");
+  /* hash.k2d: 32-byte header, then capacity x u32 */
+  const std::string hp = dir + "/hash.k2d";
+  std::unique_ptr<FILE, int (*)(FILE *)> f(fopen(hp.c_str(), "rb"), fclose);
   if (!f) return nh_set_error(NH_ERR_IO, "cannot open %s", hp.c_str());
   uint64_t hdr[4];
-  if (fread(hdr, 8, 4, f) != 4) {
-    fclose(f);
-    return nh_set_error(NH_ERR_IO, "hash.k2d: short header");
-  }
+  if (fread(hdr, 8, 4, f.get()) != 4) return nh_set_error(NH_ERR_IO, "hash.k2d: short header");
   struct stat st;
-  fstat(fileno(f), &st);
-  if ((uint64_t)st.st_size != 32 + hdr[0] * 4) {
-    fclose(f);
+  if (fstat(fileno(f.get()), &st)) return nh_set_error(NH_ERR_IO, "cannot stat %s", hp.c_str());
+  if ((uint64_t)st.st_size != 32 + hdr[0] * 4)
     return nh_set_error(NH_ERR_IO, "hash.k2d: size %lld != 32 + 4*capacity(%llu)", (long long)st.st_size,
                         (unsigned long long)hdr[0]);
-  }
-  nh_db *db = new nh_db();
-  db->info.device = device;
-  rc = parse_opts_taxo(db, opts.data(), opts.size(), taxo.data(), taxo.size());
-  if (rc) {
-    fclose(f);
-    delete db;
-    return rc;
-  }
-  const uint64_t cap = hdr[0];
-  const size_t bytes = ((cap + 31) / 32) * 128;
-  cudaError_t e = cudaMalloc(&db->d_cells, bytes);
-  if (e != cudaSuccess) {
-    fclose(f);
-    delete db;
-    return nh_set_error(NH_ERR_NOMEM, "cudaMalloc(%zu) for the hash table failed: %s", bytes,
-                        cudaGetErrorString(e));
-  }
-  db->owns_cells = true;
-  cudaMemset(db->d_cells, 0, bytes);
-  const size_t CH = 64u << 20;
-  uint8_t *stage[2] = {nullptr, nullptr};
-  cudaStream_t cs;
-  cudaStreamCreate(&cs);
-  cudaEvent_t ev[2];
-  for (int i = 0; i < 2; i++) {
-    cudaHostAlloc(&stage[i], CH, cudaHostAllocDefault);
-    cudaEventCreate(&ev[i]);
-  }
-  size_t total = cap * 4, done = 0;
-  int slot = 0;
-  rc = NH_OK;
-  while (done < total && stage[0] && stage[1]) {
-    size_t n = total - done < CH ? total - done : CH;
-    cudaEventSynchronize(ev[slot]);
-    if (fread(stage[slot], 1, n, f) != n) {
-      rc = nh_set_error(NH_ERR_IO, "hash.k2d: short read");
-      break;
-    }
-    cudaMemcpyAsync((uint8_t *)db->d_cells + done, stage[slot], n, cudaMemcpyHostToDevice, cs);
-    cudaEventRecord(ev[slot], cs);
-    done += n;
-    slot ^= 1;
-  }
-  if (!stage[0] || !stage[1]) rc = nh_set_error(NH_ERR_NOMEM, "pinned staging allocation failed");
-  cudaStreamSynchronize(cs);
-  for (int i = 0; i < 2; i++) {
-    if (stage[i]) cudaFreeHost(stage[i]);
-    cudaEventDestroy(ev[i]);
-  }
-  cudaStreamDestroy(cs);
-  fclose(f);
-  if (rc == NH_OK) {
-    e = cudaGetLastError();
-    if (e != cudaSuccess) rc = nh_set_error(NH_ERR_CUDA, "table upload failed: %s", cudaGetErrorString(e));
-  }
-  if (rc == NH_OK) rc = finish_db(db, hdr);
-  if (rc) {
-    nh_db_close(db);
-    return rc;
-  }
-  *out = db;
+  DbPtr db;
+  rc = parse_db(opts.data(), opts.size(), taxo.data(), taxo.size(), hdr, device, db);
+  if (!rc) rc = select_device(device);
+  if (!rc) rc = alloc_cells(db.get());
+  if (!rc) rc = upload_cells(f.get(), db.get());
+  if (!rc) rc = finish_db(db.get());
+  if (rc) return rc;
+  *out = db.release();
   return NH_OK;
+}
+
+/* a replica of src on `device`: the same host side, and a zeroed table for the caller to fill and then finish_db */
+static int db_replica(const nh_db *src, int device, DbPtr &db) {
+  int rc = select_device(device);
+  if (rc) return rc;
+  db.reset(new nh_db());
+  db->info = src->info;
+  db->info.device = device;
+  db->params = src->params; /* finish_db points it at the replica's own device arrays */
+  db->h_parent = src->h_parent;
+  db->h_ext = src->h_ext;
+  db->h_name = src->h_name;
+  db->h_rank = src->h_rank;
+  return alloc_cells(db.get());
 }
 
 extern "C" int nh_db_clone(const nh_db *src, int device, nh_db **out) {
   if (!src || !out) return nh_set_error(NH_ERR_INVALID, "null argument");
-  int rc = select_device(device);
+  DbPtr db;
+  int rc = db_replica(src, device, db);
   if (rc) return rc;
-  nh_db *db = new nh_db();
-  db->info = src->info;
-  db->info.device = device;
-  db->h_parent = src->h_parent;
-  db->h_ext = src->h_ext;
-  db->h_ext64 = src->h_ext64;
-  db->h_name = src->h_name;
-  db->h_rank = src->h_rank;
-  const uint64_t cap = src->info.capacity;
-  const size_t bytes = ((cap + 31) / 32) * 128;
-  cudaError_t e = cudaMalloc(&db->d_cells, bytes);
-  if (e != cudaSuccess) {
-    delete db;
-    return nh_set_error(NH_ERR_NOMEM, "cudaMalloc(%zu) for the hash table failed: %s", bytes, cudaGetErrorString(e));
-  }
-  db->owns_cells = true;
   int can = 0;
   if (cudaDeviceCanAccessPeer(&can, device, src->info.device) == cudaSuccess && can) {
     cudaError_t pe = cudaDeviceEnablePeerAccess(src->info.device, 0);
     if (pe != cudaSuccess) cudaGetLastError(); /* already enabled is fine; the copy works either way */
   }
-  e = cudaMemcpyPeer(db->d_cells, device, src->d_cells, src->info.device, bytes);
-  if (e != cudaSuccess) {
-    nh_db_close(db);
+  const cudaError_t e = cudaMemcpyPeer(db->d_cells, device, src->d_cells, src->info.device, table_bytes(src->info.capacity));
+  if (e != cudaSuccess)
     return nh_set_error(NH_ERR_CUDA, "replicating the hash table to device %d failed: %s", device, cudaGetErrorString(e));
-  }
-  const uint64_t hdr[4] = {src->info.capacity, src->info.size, src->info.key_bits, src->info.value_bits};
-  rc = finish_db(db, hdr);
-  if (rc) {
-    nh_db_close(db);
-    return rc;
-  }
-  *out = db;
+  if ((rc = finish_db(db.get()))) return rc;
+  *out = db.release();
   return NH_OK;
 }
 
@@ -510,30 +476,6 @@ struct Nccl {
 };
 }  // namespace
 
-/* an empty replica of `src` on `device`: same metadata, table allocated but not filled */
-static int db_alloc_replica(const nh_db *src, int device, nh_db **out) {
-  int rc = select_device(device);
-  if (rc) return rc;
-  nh_db *db = new nh_db();
-  db->info = src->info;
-  db->info.device = device;
-  db->h_parent = src->h_parent;
-  db->h_ext = src->h_ext;
-  db->h_ext64 = src->h_ext64;
-  db->h_name = src->h_name;
-  db->h_rank = src->h_rank;
-  const size_t bytes = ((src->info.capacity + 31) / 32) * 128;
-  cudaError_t e = cudaMalloc(&db->d_cells, bytes);
-  if (e != cudaSuccess) {
-    delete db;
-    return nh_set_error(NH_ERR_NOMEM, "cudaMalloc(%zu) for the hash table on device %d failed: %s", bytes, device,
-                        cudaGetErrorString(e));
-  }
-  db->owns_cells = true;
-  *out = db;
-  return NH_OK;
-}
-
 extern "C" int nh_db_open_multi(const char *db_dir, const int *device_ids, int n_devices, nh_db **out) {
   if (!db_dir || !device_ids || !out || n_devices < 1) return nh_set_error(NH_ERR_INVALID, "bad argument");
   for (int i = 0; i < n_devices; i++)
@@ -542,29 +484,27 @@ extern "C" int nh_db_open_multi(const char *db_dir, const int *device_ids, int n
   for (int i = 0; i < n_devices; i++) out[i] = nullptr;
   int rc = nh_db_open(db_dir, device_ids[0], &out[0]); /* the only disk read */
   if (rc || n_devices == 1) return rc;
-  auto cleanup = [&](int code) {
-    for (int i = 0; i < n_devices; i++)
-      if (out[i]) nh_db_close(out[i]), out[i] = nullptr;
-    return code;
-  };
+  std::vector<DbPtr> dbs((size_t)n_devices);
+  dbs[0].reset(out[0]);
+  out[0] = nullptr;
   for (int i = 1; i < n_devices; i++)
-    if ((rc = db_alloc_replica(out[0], device_ids[i], &out[i])) != NH_OK) return cleanup(rc);
-  const size_t bytes = ((out[0]->info.capacity + 31) / 32) * 128;
+    if ((rc = db_replica(dbs[0].get(), device_ids[i], dbs[(size_t)i])) != NH_OK) return rc;
+  const size_t bytes = table_bytes(dbs[0]->info.capacity);
   std::vector<cudaStream_t> streams((size_t)n_devices, nullptr);
-  for (int i = 0; i < n_devices; i++) {
-    cudaSetDevice(device_ids[i]);
-    cudaStreamCreateWithFlags(&streams[(size_t)i], cudaStreamNonBlocking);
-  }
+  cudaError_t e = cudaSuccess;
+  for (int i = 0; i < n_devices && e == cudaSuccess; i++)
+    if ((e = cudaSetDevice(device_ids[i])) == cudaSuccess)
+      e = cudaStreamCreateWithFlags(&streams[(size_t)i], cudaStreamNonBlocking);
   int how = 0;
   Nccl nccl;
-  if (nccl.load()) {
+  if (e == cudaSuccess && nccl.load()) {
     std::vector<nccl_comm_t> comms((size_t)n_devices, nullptr);
     int nr = nccl.CommInitAll(comms.data(), n_devices, device_ids);
     if (nr == 0) {
       nccl.GroupStart();
       for (int i = 0; i < n_devices && nr == 0; i++) {
         cudaSetDevice(device_ids[i]);
-        nr = nccl.Broadcast(out[0]->d_cells, out[i]->d_cells, bytes, 1 /* ncclUint8 */, 0, comms[(size_t)i], streams[(size_t)i]);
+        nr = nccl.Broadcast(dbs[0]->d_cells, dbs[(size_t)i]->d_cells, bytes, 1 /* ncclUint8 */, 0, comms[(size_t)i], streams[(size_t)i]);
       }
       const int ge = nccl.GroupEnd();
       if (nr == 0) nr = ge;
@@ -578,10 +518,9 @@ extern "C" int nh_db_open_multi(const char *db_dir, const int *device_ids, int n
     if (nr == 0) how = 1;
     else cudaGetLastError(); /* fall through to the peer copies */
   }
-  if (!how) {
+  if (e == cudaSuccess && !how) {
     /* binomial tree of peer copies: round r doubles the number of replicas (3 rounds for 8 GPUs),
      * every copy of a round on its own stream so they run side by side over NVSwitch */
-    cudaError_t e = cudaSuccess;
     for (int have = 1; have < n_devices && e == cudaSuccess; have *= 2) {
       for (int i = 0; i < have && have + i < n_devices; i++) {
         const int src = i, dst = have + i;
@@ -589,7 +528,8 @@ extern "C" int nh_db_open_multi(const char *db_dir, const int *device_ids, int n
         cudaSetDevice(device_ids[dst]);
         if (cudaDeviceCanAccessPeer(&can, device_ids[dst], device_ids[src]) == cudaSuccess && can)
           if (cudaDeviceEnablePeerAccess(device_ids[src], 0) != cudaSuccess) cudaGetLastError();
-        e = cudaMemcpyPeerAsync(out[dst]->d_cells, device_ids[dst], out[src]->d_cells, device_ids[src], bytes, streams[(size_t)dst]);
+        e = cudaMemcpyPeerAsync(dbs[(size_t)dst]->d_cells, device_ids[dst], dbs[(size_t)src]->d_cells, device_ids[src], bytes,
+                                streams[(size_t)dst]);
         if (e != cudaSuccess) break;
       }
       for (int i = 0; i < have && have + i < n_devices; i++) {
@@ -598,22 +538,19 @@ extern "C" int nh_db_open_multi(const char *db_dir, const int *device_ids, int n
         if (e == cudaSuccess) e = se;
       }
     }
-    if (e != cudaSuccess) {
-      for (auto st : streams) cudaStreamDestroy(st);
-      return cleanup(nh_set_error(NH_ERR_CUDA, "replicating the hash table failed: %s", cudaGetErrorString(e)));
-    }
     how = 2;
   }
-  for (int i = 0; i < n_devices; i++) {
-    cudaSetDevice(device_ids[i]);
-    cudaStreamDestroy(streams[(size_t)i]);
-  }
-  const uint64_t hdr[4] = {out[0]->info.capacity, out[0]->info.size, out[0]->info.key_bits, out[0]->info.value_bits};
+  for (int i = 0; i < n_devices; i++)
+    if (streams[(size_t)i]) {
+      cudaSetDevice(device_ids[i]);
+      cudaStreamDestroy(streams[(size_t)i]);
+    }
+  if (e != cudaSuccess) return nh_set_error(NH_ERR_CUDA, "replicating the hash table failed: %s", cudaGetErrorString(e));
   for (int i = 1; i < n_devices; i++) {
-    cudaSetDevice(device_ids[i]);
-    if ((rc = finish_db(out[i], hdr)) != NH_OK) return cleanup(rc);
-    out[i]->info.replicated_by = how;
+    if ((rc = finish_db(dbs[(size_t)i].get())) != NH_OK) return rc;
+    dbs[(size_t)i]->info.replicated_by = how;
   }
+  for (int i = 0; i < n_devices; i++) out[i] = dbs[(size_t)i].release();
   return NH_OK;
 }
 
@@ -627,12 +564,13 @@ extern "C" const uint32_t *nh_db_device_cells(const nh_db *db) { return db ? db-
 
 extern "C" void nh_db_close(nh_db *db) {
   if (!db) return;
-  cudaSetDevice(db->info.device);
-  if (db->owns_cells && db->d_cells) cudaFree(db->d_cells);
-  if (db->d_parent) cudaFree(db->d_parent);
-  if (db->d_ext) cudaFree(db->d_ext);
-  if (db->d_huge) cudaFree(db->d_huge);
-  if (db->d_filter) cudaFree(db->d_filter);
+  /* a handle that failed before its device work owns no device memory, and closing it makes no CUDA call */
+  void *owned[] = {db->owns_cells ? db->d_cells : nullptr, db->d_parent, db->d_ext, db->d_huge, db->d_filter};
+  for (void *p : owned)
+    if (p) {
+      cudaSetDevice(db->info.device);
+      cudaFree(p);
+    }
   delete db;
 }
 

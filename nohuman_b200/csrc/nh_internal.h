@@ -36,7 +36,6 @@ struct nh_db {
   uint32_t n_filter_blocks = 0; /* 0 until the filter is built */
   uint32_t *d_huge = nullptr; /* global-memory taxon table for units with more distinct taxa than shared memory holds */
   std::vector<uint32_t> h_parent, h_ext;
-  std::vector<uint64_t> h_ext64;
   std::vector<std::string> h_name, h_rank; /* taxo.k2d name / rank strings per node (reports) */
   int sm_count = 0;
 };
@@ -100,6 +99,9 @@ void nh_pack_range(const uint8_t *bases, const uint64_t *offsets, uint64_t total
 
 int nh_set_error(int code, const char *fmt, ...);
 int nh_db_build_filter(nh_db *db); /* after the cells are on the device (every open path; the synthetic builder calls it itself) */
+/* zeroed table of `capacity` cells for the synthetic builder (nh_synth.cu), which fills it and builds the filter */
+int nh_db_create_empty(const void *opts, size_t opts_len, const void *taxo, size_t taxo_len, uint64_t capacity, int device,
+                       nh_db **out);
 int nh_session_create_ex(nh_db *db, const nh_params_t *params, bool need_lookups, nh_session **out);
 int nh_resolve_db_dir(const char *db_dir, std::string &out);
 

@@ -1284,7 +1284,7 @@ static bool write_report(const char *path, const nh_db *db, const std::vector<ui
     if (!named) fr.rank_depth++;
     std::string rs(1, fr.code);
     if (fr.rank_depth != 0) rs += std::to_string(fr.rank_depth);
-    line(clade[fr.id], call_counts[fr.id], rs, db->h_ext64[fr.id], db->h_name[fr.id], fr.depth);
+    line(clade[fr.id], call_counts[fr.id], rs, db->h_ext[fr.id], db->h_name[fr.id], fr.depth);
     std::vector<uint32_t> ch = kids[fr.id];
     std::stable_sort(ch.begin(), ch.end(), [&](uint32_t a, uint32_t b) { return clade[a] > clade[b]; });
     for (auto it = ch.rbegin(); it != ch.rend(); ++it) stack.push_back({*it, fr.code, fr.rank_depth, fr.depth + 1});

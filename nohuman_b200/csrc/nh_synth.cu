@@ -112,10 +112,6 @@ k_insert_tiles(const NhDbParams db, uint32_t *cells, const NhBatchPtrs b, uint64
   if (lane == 0 && claimed) atomicAdd(size_counter, (unsigned long long)claimed);
 }
 
-/* defined in nh_capi.cu */
-int nh_db_create_empty(const void *opts, size_t opts_len, const void *taxo, size_t taxo_len,
-                       uint64_t capacity, int device, nh_db **out);
-
 extern "C" int nh_synth_build_db(const void *opts, size_t opts_len, const void *taxo,
                                  size_t taxo_len, const uint32_t *leaf_taxa, int n_leaves,
                                  const nh_synth_db_params_t *p, int device, nh_db **out,
