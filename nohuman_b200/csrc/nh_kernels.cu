@@ -473,11 +473,9 @@ __device__ __forceinline__ void ld_sector(const uint32_t *p, uint32_t (&c)[8]) {
                : "l"(p));
 }
 
-__device__ __forceinline__ uint32_t cht_get(const NhDbParams &db, uint64_t key) {
-  const uint64_t h = nh_fmix64(key);
-  if (db.min_hash && h < db.min_hash) return 0;
-  const uint32_t ckey = (uint32_t)(h >> (32u + db.value_bits));
-  uint64_t idx = nh_fastmod(h, db.capacity, db.mod_m, db.mod_sh1, db.mod_sh2);
+/* the probe chain of compacted key ckey from cell idx on: the value of the first cell that is empty or holds ckey,
+ * 0 after a whole table without either.  64-bit throughout, so it walks any distance. */
+__device__ __forceinline__ uint32_t cht_walk(const NhDbParams &db, uint64_t idx, uint32_t ckey) {
   uint64_t inspected = 0;
   for (;;) {
     const uint64_t sbase = idx & ~7ULL;
@@ -499,6 +497,13 @@ __device__ __forceinline__ uint32_t cht_get(const NhDbParams &db, uint64_t key) 
     idx = sbase + 8;
     if (idx >= db.capacity) idx = 0;
   }
+}
+
+__device__ __forceinline__ uint32_t cht_get(const NhDbParams &db, uint64_t key) {
+  const uint64_t h = nh_fmix64(key);
+  if (db.min_hash && h < db.min_hash) return 0;
+  return cht_walk(db, nh_fastmod(h, db.capacity, db.mod_m, db.mod_sh1, db.mod_sh2),
+                  (uint32_t)(h >> (32u + db.value_bits)));
 }
 
 __global__ void __launch_bounds__(256)
@@ -1058,9 +1063,15 @@ k_stream_classify(const NhDbParams db, const NhBatchPtrs b, const NhScoreParams 
   const uint32_t last_sector = n_sectors - 1u;
   /* cells of the last sector that exist (the allocation is zero-padded past the table's end) */
   const uint32_t last_range = (db.capacity & 7ULL) ? (1u << (uint32_t)(db.capacity & 7ULL)) - 1u : 0xFFu;
-  /* probe-chain guard for a table without any empty cell (never a real database) */
-  /* FILTER kernels keep bit 31 of the lookup state for NH_AUX_FILTER, and the cell a continuation starts at in
-   * the top value_bits (>= 5, nh_db_build_filter) bits of its compacted key */
+  /* The visit count of a chain lives in 16 bits of its state (15 in the FILTER kernels, which keep bit 31 for
+   * NH_AUX_FILTER and the cell a continuation starts at in the top value_bits (>= 5, nh_db_build_filter) bits of
+   * its compacted key).  A chain that reaches max_visits is not a miss: every unit of the group is marked
+   * overflowed, like a unit with more taxa than a lane table holds, and k_score_big classifies them again with
+   * cht_get, which walks any distance and still ends on a table without any empty cell (one constant store keeps
+   * the probe round's code as it was).  EMIT kernels also need the lookup's own taxon for
+   * the per-read output, so there the lane walks the rest of the chain itself with cht_walk.  Only tables built at a
+   * load close to 1 have runs that long (about 262 K cells when walking sectors in the FILTER kernels, 524 K
+   * otherwise), and the common branch gains nothing. */
   const uint32_t max_visits = FILTER ? (n_sectors + 1u < 0x7FFEu ? n_sectors + 1u : 0x7FFEu) : (n_sectors + 1u < 0xFFFFu ? n_sectors + 1u : 0xFFFFu);
   const uint32_t last_block = FILTER ? sp.n_filter_blocks - 1u : 0u;
   const uint32_t ck_bits = 32u - db.value_bits;
@@ -1150,6 +1161,7 @@ k_stream_classify(const NhDbParams db, const NhBatchPtrs b, const NhScoreParams 
                 done = true; /* the key is not in the block and the chain ends in it: a miss */
               } else if (visits >= max_visits) {
                 done = true;
+                atomicOr(&sm.overflow, FULL_MASK); /* every unit of the group: k_score_big walks the rest */
               } else if (maybe) { /* to the table, at the cell the chain has reached */
                 f_aux = (f_aux & 0xFFFFu) | (visits << 16);
                 f_unit = f_unit * 4u + (st >> 3);
@@ -1172,7 +1184,8 @@ k_stream_classify(const NhDbParams db, const NhBatchPtrs b, const NhScoreParams 
                 done = true;
                 result = (uint32_t)state;
               } else if (visits >= max_visits) {
-                done = true; /* went round a table without an empty cell */
+                done = true;
+                atomicOr(&sm.overflow, FULL_MASK); /* every unit of the group: k_score_big walks the rest */
               } else {
                 f_aux = (f_aux & 0xFFFFu) | (visits << 16);
                 f_unit = f_unit == last_sector ? 0u : f_unit + 1u;
@@ -1194,7 +1207,9 @@ k_stream_classify(const NhDbParams db, const NhBatchPtrs b, const NhScoreParams 
           } else {
             const uint32_t visits = (f_aux >> 16) + 1u;
             if (visits >= max_visits) {
-              done = true; /* went round a table without an empty cell */
+              done = true;
+              if (EMIT) result = cht_walk(db, (uint64_t)f_unit * 8ULL + f_start, f_ckey);
+              else atomicOr(&sm.overflow, FULL_MASK); /* every unit of the group: k_score_big walks the rest */
             } else {
               f_aux = (f_aux & 0xFFFFu) | (visits << 16);
               f_unit = f_unit == last_sector ? 0u : f_unit + 1u;
