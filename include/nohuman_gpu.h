@@ -78,7 +78,9 @@ typedef struct {
   uint64_t max_batch_seqs;    /* session capacity; 0 selects max_batch_bases/64 */
   int32_t emit_runs;          /* 1: keep per-sequence (taxid, k-mer count) runs for nh_last_batch_runs
                                  (kraken2's per-read output, --output; costs 5 B per lookup of D2H) */
-  int32_t reserved;
+  int32_t gpu_gzip;           /* 1: gzip output ('g') of nh_run_files / nh_run_files_multi is deflated on the
+                                 sessions' GPUs (nh_bgzf_compress's members); 0: zlib level 6 on -t host threads.
+                                 Other formats ignore it. */
 } nh_params_t;
 
 typedef struct {
@@ -112,9 +114,9 @@ typedef struct {
   double busy_stage_s;     /* interleaving mates into the pinned transfer buffers (2 threads per GPU) */
   double busy_classify_s;  /* inside nh_classify_batch: H2D, kernels, D2H (same threads) */
   double busy_serialise_s; /* re-serialising kept records, per-read output lines (same threads) */
-  double busy_compress_s;  /* output compression (-t threads) */
+  double busy_compress_s;  /* output compression (-t threads; with gpu_gzip, the GPU deflater threads) */
   double busy_write_s;     /* ordered writes to the output files (1 thread) */
-  int32_t threads_inflate, threads_compress;
+  int32_t threads_inflate, threads_compress; /* threads_compress: -t, or one GPU deflater thread per GPU */
 } nh_run_stats_t;
 
 /* ------------------------------------------------------------------ */
@@ -240,6 +242,17 @@ int nh_run_files_multi(nh_session *const *sessions, int n_sessions, const nh_fil
  * supplied by the caller. */
 int nh_debug_rewrite_files(const nh_files_t *files, const uint8_t *keep, const uint32_t *call_ext,
                            uint64_t n_units, int threads, nh_run_stats_t *stats);
+
+/* BGZF compression on the GPU: in[0..n) becomes gzip members of 0xff00 input bytes each (byte i goes into
+ * member i / 0xff00), as the gzip output of nh_run_files is cut, without bgzip's empty end-of-file member.
+ * Every member carries the 'BC' subfield with its size and holds one deflate block (dynamic Huffman codes,
+ * or stored when that is not smaller), so no member exceeds 65 311 bytes.  The same input gives the same
+ * bytes on every call and every GPU.  out_cap must be at least ceil(n / 0xff00) * 65536
+ * (NH_ERR_CAPACITY otherwise); *out_len gets the bytes written. */
+int nh_bgzf_compress(int device, const uint8_t *in, size_t n, uint8_t *out, size_t out_cap, size_t *out_len);
+/* Device time of nh_bgzf_compress's kernels for one batch of n bytes (1 byte to 1 GiB) already on the device:
+ * mean over `iters` launches after one warm-up, in seconds. */
+int nh_bench_bgzf(int device, const uint8_t *in, size_t n, int iters, double *out_seconds);
 
 /* Pinned host memory for callers that want true async copies. */
 void *nh_host_alloc(size_t bytes);

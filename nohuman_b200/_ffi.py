@@ -48,7 +48,7 @@ class Params(C.Structure):
         ("confidence", C.c_double), ("minimum_hit_groups", C.c_int32), ("paired", C.c_int32),
         ("keep_human", C.c_int32), ("threads", C.c_int32),
         ("max_batch_bases", C.c_uint64), ("max_batch_seqs", C.c_uint64),
-        ("emit_runs", C.c_int32), ("reserved", C.c_int32),
+        ("emit_runs", C.c_int32), ("gpu_gzip", C.c_int32),
     ]
 
 
@@ -113,6 +113,8 @@ SYMBOLS = {
     "nh_debug_rewrite_files": (_i32, [C.POINTER(Files), _vp, _vp, _u64, _i32, C.POINTER(RunStats)]),
     "nh_session_stream": (_vp, [_vp]),
     "nh_last_batch_runs": (_i32, [_vp, _u64, _vp, _vp, _vp, _u64, C.POINTER(_u64)]),
+    "nh_bgzf_compress": (_i32, [_i32, _vp, C.c_size_t, _vp, C.c_size_t, C.POINTER(C.c_size_t)]),
+    "nh_bench_bgzf": (_i32, [_i32, _vp, C.c_size_t, _i32, C.POINTER(C.c_double)]),
     "nh_host_alloc": (_vp, [C.c_size_t]),
     "nh_host_free": (None, [_vp]),
     "nh_debug_minimizers": (_i32, [_vp, _vp, _vp, _u64, _vp, _vp, _vp]),

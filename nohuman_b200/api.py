@@ -83,6 +83,27 @@ def pack_reads(bases: np.ndarray, offsets: np.ndarray, threads: int = 1):
     return codes, valid, poff
 
 
+BGZF_INPUT = 0xFF00  # input bytes per BGZF member
+
+
+def bgzf_compress(data: bytes, device: int = 0) -> bytes:
+    """BGZF members of `data` (0xff00 input bytes each, no end-of-file member), deflated on `device`
+    (nh_bgzf_compress).  gzip.decompress() reads the result."""
+    n = len(data)
+    cap = -(-n // BGZF_INPUT) * 65536
+    out = np.empty(max(cap, 1), np.uint8)  # not zero-filled: only the bytes written are read back
+    got = C.c_size_t()
+    check(lib().nh_bgzf_compress(int(device), data, n, out.ctypes.data, cap, C.byref(got)))
+    return C.string_at(out.ctypes.data, got.value)
+
+
+def bgzf_kernel_seconds(data: bytes, device: int = 0, iters: int = 10) -> float:
+    """Device time of the BGZF kernels for `data` in one batch (nh_bench_bgzf), mean of `iters` launches."""
+    t = C.c_double()
+    check(lib().nh_bench_bgzf(int(device), data, len(data), int(iters), C.byref(t)))
+    return t.value
+
+
 class Database:
     """A kraken2 database (hash.k2d / opts.k2d / taxo.k2d) resident in HBM."""
 
@@ -165,7 +186,8 @@ class Session:
 
     def __init__(self, db: Database, confidence: float = 0.0, paired: bool = False,
                  keep_human: bool = False, minimum_hit_groups: int = 2, threads: int = 1,
-                 max_batch_bases: int = 0, max_batch_seqs: int = 0, emit_runs: bool = False):
+                 max_batch_bases: int = 0, max_batch_seqs: int = 0, emit_runs: bool = False,
+                 gpu_gzip: bool = False):
         p = Params()
         p.confidence = float(confidence)
         p.minimum_hit_groups = int(minimum_hit_groups)
@@ -175,6 +197,7 @@ class Session:
         p.max_batch_bases = int(max_batch_bases)
         p.max_batch_seqs = int(max_batch_seqs)
         p.emit_runs = int(emit_runs)
+        p.gpu_gzip = int(gpu_gzip)  # gzip output of run_files / run_files_multi deflated on the GPU
         self.paired = bool(paired)
         self.db = db
         self._h = C.c_void_p()

@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <functional>
 #include <string>
 #include <vector>
 
@@ -96,6 +97,40 @@ struct nh_session {
  * non-temporal stores when the CPU has it */
 void nh_pack_range(const uint8_t *bases, const uint64_t *offsets, uint64_t total_bases, uint64_t s0, uint64_t s1, uint8_t *codes,
                    uint32_t *valid, const uint32_t *poff);
+
+/* nh_deflate.cu: BGZF compression on one GPU with its own stream, device buffers and pinned staging for a
+ * batch of up to batch_bytes of input.  compress() cuts every block into 0xff00-byte members as the zlib
+ * path does and returns each block's members, one string per block, or hands them in order to a sink; larger
+ * inputs go in several rounds.
+ * Not thread-safe: one per thread. */
+class GpuDeflater {
+ public:
+  typedef std::pair<const uint8_t *, size_t> Span;
+  /* receives the members in order: (block index, bytes, length), one call per member */
+  typedef std::function<void(size_t, const uint8_t *, size_t)> Sink;
+  static constexpr size_t kBatchBytes = size_t(32) << 20;
+  GpuDeflater() = default;
+  GpuDeflater(const GpuDeflater &) = delete;
+  GpuDeflater &operator=(const GpuDeflater &) = delete;
+  ~GpuDeflater();
+  int open(int device, size_t batch_bytes = kBatchBytes); /* NH_OK or an nh_status with nh_last_error() set */
+  int compress(const std::vector<Span> &blocks, std::vector<std::string> &out);
+  int compress(const std::vector<Span> &blocks, const Sink &sink);
+  /* device time of the kernels for one batch of `n` bytes (already cut into members), mean of `iters` */
+  int time_kernels(const uint8_t *in, size_t n, int iters, double *seconds);
+
+ private:
+  int launch(size_t n_members);
+  int run(size_t bytes, size_t n_members);
+  int device_ = -1;
+  size_t batch_ = 0, max_members_ = 0;
+  cudaStream_t stream_ = nullptr;
+  uint8_t *d_in_ = nullptr, *d_slots_ = nullptr, *d_out_ = nullptr;
+  uint8_t *h_in_ = nullptr, *h_out_ = nullptr;
+  uint2 *d_members_ = nullptr, *h_members_ = nullptr;
+  uint32_t *d_scratch_ = nullptr, *d_sizes_ = nullptr;
+  uint64_t *d_offs_ = nullptr, *h_offs_ = nullptr;
+};
 
 int nh_set_error(int code, const char *fmt, ...);
 int nh_db_build_filter(nh_db *db); /* after the cells are on the device (every open path; the synthetic builder calls it itself) */

@@ -1027,10 +1027,14 @@ struct Block {
   bool done = false;
 };
 
+/* Compresses blocks on `threads` host threads, or, given GPUs, on one deflater thread per GPU that takes
+ * every waiting block up to GpuDeflater::kBatchBytes at a time; the flusher writes them in order. */
 class BlockWriter {
  public:
-  BlockWriter(OutputFile *files, int n_files, int threads, StageClock *clk) : files_(files), n_files_(n_files), clk_(clk) {
-    int n = threads < 1 ? 1 : threads;
+  BlockWriter(OutputFile *files, int n_files, int threads, const std::vector<int> &gpus, StageClock *clk)
+      : files_(files), n_files_(n_files), clk_(clk) {
+    for (int dev : gpus) workers_.emplace_back([this, dev] { gpu_work(dev); });
+    const int n = gpus.empty() ? (threads < 1 ? 1 : threads) : 0;
     for (int i = 0; i < n; i++) workers_.emplace_back([this] { work(); });
     flusher_ = std::thread([this] { flush(); });
   }
@@ -1058,8 +1062,54 @@ class BlockWriter {
     flusher_.join();
     return ok_;
   }
+  /* the first GPU deflater failure (NH_OK if none) and its message */
+  int error(std::string &msg) const {
+    msg = err_msg_;
+    return err_code_;
+  }
 
  private:
+  void gpu_work(int device) {
+    GpuDeflater gd;
+    int rc = gd.open(device);
+    std::string msg = rc ? nh_last_error() : "";
+    for (;;) {
+      std::vector<std::shared_ptr<Block>> batch;
+      {
+        std::unique_lock<std::mutex> lk(m_);
+        cv_.wait(lk, [&] { return !todo_.empty() || closing_; });
+        if (todo_.empty()) return;
+        size_t bytes = 0;
+        while (!todo_.empty() && (batch.empty() || bytes + todo_.front()->raw.size() <= GpuDeflater::kBatchBytes)) {
+          bytes += todo_.front()->raw.size();
+          batch.push_back(todo_.front());
+          todo_.pop_front();
+        }
+      }
+      if (rc == NH_OK) {
+        Busy busy(clk_, ST_COMPRESS);
+        std::vector<GpuDeflater::Span> spans;
+        for (auto &b : batch) spans.emplace_back((const uint8_t *)b->raw.data(), b->raw.size());
+        std::vector<std::string> packed;
+        rc = gd.compress(spans, packed);
+        if (rc != NH_OK)
+          msg = nh_last_error();
+        else
+          for (size_t i = 0; i < batch.size(); i++) batch[i]->packed = std::move(packed[i]);
+      }
+      std::lock_guard<std::mutex> lk(m_);
+      if (rc != NH_OK) {
+        ok_ = false;
+        if (err_code_ == NH_OK) err_code_ = rc, err_msg_ = msg;
+      }
+      for (auto &b : batch) {
+        b->raw.clear();
+        b->raw.shrink_to_fit();
+        b->done = true;
+      }
+      cv_.notify_all();
+    }
+  }
   void work() {
     for (;;) {
       std::shared_ptr<Block> b;
@@ -1112,6 +1162,8 @@ class BlockWriter {
   std::thread flusher_;
   bool closing_ = false;
   bool ok_ = true;
+  int err_code_ = NH_OK;
+  std::string err_msg_;
 };
 
 /* ------------------------------------------------------------------ */
@@ -1571,8 +1623,13 @@ static int run_pipeline(const Decider &dec, const nh_files_t *files, nh_run_stat
       done_cv.notify_all();
     });
 
-  /* writer (this thread): batches in id order */
-  BlockWriter bw(outs, nf, threads, &clock);
+  /* writer (this thread): batches in id order; gzip output is deflated on the sessions' GPUs on request */
+  std::vector<int> deflate_gpus;
+  if (dec.params.gpu_gzip && fmt == 'g')
+    for (const nh_db *db : dec.dbs)
+      if (std::find(deflate_gpus.begin(), deflate_gpus.end(), db->info.device) == deflate_gpus.end())
+        deflate_gpus.push_back(db->info.device);
+  BlockWriter bw(outs, nf, threads, deflate_gpus, &clock);
   uint64_t want = 0, total_units = 0, n_classified = 0, total_bases = 0;
   std::string pend[2];
   for (;;) {
@@ -1643,6 +1700,8 @@ static int run_pipeline(const Decider &dec, const nh_files_t *files, nh_run_stat
     fail_msg = std::string("writing ") + files->kraken_report + " failed";
   }
   if (failed) return nh_set_error(NH_ERR_IO, "%s", fail_msg.c_str());
+  std::string deflate_msg;
+  if (const int rc = bw.error(deflate_msg)) return nh_set_error(rc, "%s", deflate_msg.c_str());
   if (!wrote) return nh_set_error(NH_ERR_IO, "writing %s failed", outs[0].path().c_str());
   if (stats) {
     stats->total = total_units;
@@ -1658,7 +1717,7 @@ static int run_pipeline(const Decider &dec, const nh_files_t *files, nh_run_stat
     stats->busy_compress_s = 1e-9 * (double)clock.ns[ST_COMPRESS];
     stats->busy_write_s = 1e-9 * (double)clock.ns[ST_WRITE];
     stats->threads_inflate = readers[0].inflate_threads() + (paired ? readers[1].inflate_threads() : 0);
-    stats->threads_compress = outs[0].parallel() ? threads : 0;
+    stats->threads_compress = !outs[0].parallel() ? 0 : deflate_gpus.empty() ? threads : (int)deflate_gpus.size();
   }
   return NH_OK;
 }

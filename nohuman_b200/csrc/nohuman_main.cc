@@ -384,6 +384,7 @@ static void usage() {
        "  -r, --kraken-report <FILE> Write the Kraken2 report with aggregate counts/clade to file\n"
        "      --gpu <ID>             First CUDA device to use [default: 0]\n"
        "      --gpus <N|all>         Number of GPUs: read batches are sharded, the database is replicated [default: 1]\n"
+       "      --gpu-gzip             Compress gzip output (-F g) on the GPUs instead of the host threads\n"
        "  -v, --verbose              Set the logging level to verbose\n"
        "  -h, --help                 Print help\n"
        "  -V, --version              Print version");
@@ -397,10 +398,10 @@ int main(int argc, char **argv) {
                           {"human", 0, 0, 'H'},        {"conf", 1, 0, 'C'},          {"kraken-output", 1, 0, 'k'},
                           {"kraken-report", 1, 0, 'r'}, {"verbose", 0, 0, 'v'},      {"help", 0, 0, 'h'},
                           {"version", 0, 0, 'V'},      {"gpu", 1, 0, 3},             {"plan", 0, 0, 4},
-                          {"gpus", 1, 0, 5},
+                          {"gpus", 1, 0, 5},           {"gpu-gzip", 0, 0, 6},
                           {0, 0, 0, 0}};
   std::string out1, out2, db, db_version, kraken_output, kraken_report, err;
-  bool check = false, download = false, list = false, human = false, plan = false;
+  bool check = false, download = false, list = false, human = false, plan = false, gpu_gzip = false;
   int out_type = 0, gpu = 0, gpus = 1;
   long threads = 1;
   double conf = 0.0;
@@ -437,6 +438,7 @@ int main(int argc, char **argv) {
       case 3: gpu = atoi(optarg); break;
       case 5: gpus = !strcmp(optarg, "all") ? -1 : atoi(optarg); break;
       case 4: plan = true; break; /* hidden: print what would run (database, format, outputs) and exit */
+      case 6: gpu_gzip = true; break;
       default: return 2;
     }
   std::vector<std::string> input(argv + optind, argv + argc);
@@ -518,8 +520,10 @@ int main(int argc, char **argv) {
   if (paired && out2.empty()) out2 = default_output(input[1], fmt);
 
   if (plan) {
-    printf("db=%s\nversion=%s\nformat=%c\nout1=%s\nout2=%s\npaired=%d\nkeep_human=%d\nconfidence=%.17g\nthreads=%ld\n",
-           db_path.c_str(), version.c_str(), fmt, out1.c_str(), out2.c_str(), (int)paired, (int)human, conf, threads);
+    printf("db=%s\nversion=%s\nformat=%c\nout1=%s\nout2=%s\npaired=%d\nkeep_human=%d\nconfidence=%.17g\nthreads=%ld\n"
+           "gpu_gzip=%d\n",
+           db_path.c_str(), version.c_str(), fmt, out1.c_str(), out2.c_str(), (int)paired, (int)human, conf, threads,
+           (int)gpu_gzip);
     return 0;
   }
   /* more GPUs: the table is read from disk once and broadcast (NCCL over NVLink, else peer copies);
@@ -540,6 +544,7 @@ int main(int argc, char **argv) {
   p.paired = paired;
   p.keep_human = human;
   p.threads = (int)threads;
+  p.gpu_gzip = gpu_gzip;
   p.max_batch_bases = 1u << 20; /* parameter carrier only: nh_run_files sizes its own sessions */
   p.max_batch_seqs = 1u << 12;
   std::vector<nh_session *> sessions;

@@ -205,3 +205,28 @@ def synth_genome(device: int, genome_seed: int, start: int, n: int) -> np.ndarra
     out = np.empty(n, np.uint8)
     check(_lib().nh_synth_genome(device, genome_seed, start, n, out.ctypes.data))
     return out
+
+
+def fastq_corpus(n_bytes: int, seed: int = 0, random_quals: bool = False, read_len: int = 150) -> bytes:
+    """Seeded FASTQ text of n_bytes (the last record cut short), laid out as the file pipeline writes kept
+    reads: `@r<9-digit id>/1` headers, bases from ACGT with 1 % N, `+`, and qualities that are all `I` as
+    in tools/file_pipeline_bench.py, or uniformly random Phred 2..41 (random_quals).  The corpus of the
+    GPU gzip ratio checks and of tools/gzip_bench.py."""
+    rng = np.random.default_rng(seed)
+    hdr_len = len(b"@r000000000/1\n")
+    rec_len = hdr_len + 2 * read_len + 4
+    n = max(1, -(-n_bytes // rec_len))
+    rec = np.empty((n, rec_len), np.uint8)
+    rec[:, :hdr_len] = np.frombuffer(b"@r000000000/1\n", np.uint8)
+    idx = np.arange(n)
+    for d in range(9):
+        rec[:, 2 + 8 - d] = 48 + (idx // 10 ** d) % 10
+    seq = np.frombuffer(b"ACGT", np.uint8)[rng.integers(0, 4, size=(n, read_len))]
+    seq[rng.random((n, read_len)) < 0.01] = ord("N")
+    o = hdr_len
+    rec[:, o:o + read_len] = seq
+    rec[:, o + read_len:o + read_len + 3] = np.frombuffer(b"\n+\n", np.uint8)
+    q = rec[:, o + read_len + 3:o + 2 * read_len + 3]
+    q[:] = rng.integers(33 + 2, 33 + 42, size=q.shape) if random_quals else ord("I")
+    rec[:, -1] = ord("\n")
+    return rec.tobytes()[:n_bytes]

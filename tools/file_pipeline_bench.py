@@ -4,7 +4,11 @@ FASTQ (50 % genome-derived), gzip in / gzip out, against the synthetic HPRC.r2-s
 Wall clock of the whole CLI process and of the pipeline alone, busy seconds per host stage, and a check of the
 OUTPUT BYTES against what the CPU oracle says must be kept.
 
-    python tools/file_pipeline_bench.py [--pairs 10000000] [--threads 16] [--capacity-log2 31] [--gpus 1]
+    python tools/file_pipeline_bench.py [--pairs 10000000] [--threads 16[,4...]] [--capacity-log2 31] [--gpus 1]
+                                        [--gpu-gzip]
+
+--threads takes a comma-separated list: every variant runs at each count.  --gpu-gzip deflates the gzip
+output on the GPU (nohuman --gpu-gzip) instead of on the host threads.
 """
 import argparse
 import hashlib
@@ -65,12 +69,14 @@ def sha_of_rows(rec2d, keep):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--pairs", type=int, default=10_000_000)
-    ap.add_argument("--threads", type=int, default=os.cpu_count() or 16)
+    ap.add_argument("--threads", default=str(os.cpu_count() or 16))
     ap.add_argument("--capacity-log2", type=int, default=31)
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--variants", default="gz-gz,bgz-gz,plain-plain,gz-plain,bgz-plain,plain-gz")
     ap.add_argument("--tmp", default=None)
+    ap.add_argument("--gpu-gzip", action="store_true")
     args = ap.parse_args()
+    thread_counts = [int(t) for t in args.threads.split(",")]
     import torch
     from nohuman_b200 import synth
     from oracle import k2oracle  # the checker of the output bytes; not in any timed region
@@ -119,19 +125,20 @@ def main():
         # blocked gzip (BGZF: what bgzip / bcl2fastq / this library write) of the same reads, made with the host-only hook
         from nohuman_b200.api import rewrite_files
         rewrite_files(np.ones(args.pairs, np.uint8), np.zeros(args.pairs, np.uint32), p1, b1, p2, b2, out_format="g",
-                      threads=args.threads)
+                      threads=max(thread_counts))
     cli = os.path.join(ROOT, "nohuman_b200", "bin", "nohuman")
     rows = []
     gbp = args.pairs * 2 * L / 1e9
     ins = {"plain": (p1, p2), "gz": (p1 + ".gz", p2 + ".gz"), "bgz": (b1, b2)}
-    for v in variants:
+    for v, threads in [(v, t) for t in thread_counts for v in variants]:
         vin, vout = v.split("-")
         a, b = ins[vin]
         fmt = "g" if vout == "gz" else "u"
         o1, o2 = os.path.join(d, "o1"), os.path.join(d, "o2")
         t0 = time.perf_counter()
-        r = subprocess.run([cli, "-v", "--db", db_dir, "-t", str(args.threads), "--conf", "0.5", "-F", fmt, "-o", o1, "-O", o2,
-                            "--gpus", str(args.gpus), a, b], capture_output=True, text=True)
+        r = subprocess.run([cli, "-v", "--db", db_dir, "-t", str(threads), "--conf", "0.5", "-F", fmt, "-o", o1, "-O", o2,
+                            "--gpus", str(args.gpus), *(["--gpu-gzip"] if args.gpu_gzip else []), a, b],
+                           capture_output=True, text=True)
         dt = time.perf_counter() - t0
         assert r.returncode == 0, r.stderr
         dbg = [ln.split("] ", 1)[1] for ln in r.stderr.splitlines() if "DEBUG" in ln]
@@ -143,6 +150,7 @@ def main():
         got1 = sha_of_stream(["gzip", "-dc", o1] if fmt == "g" else ["cat", o1])
         got2 = sha_of_stream(["gzip", "-dc", o2] if fmt == "g" else ["cat", o2])
         rows.append({"variant": f"{vin} in, {vout} out" + (" (configs[1])" if v == "gz-gz" else ""), "gpus": args.gpus,
+                     "threads": threads, "gpu_gzip": bool(args.gpu_gzip and fmt == "g"),
                      "seconds": round(dt, 2), "gbp_s": round(gbp / dt, 3),
                      "pipeline_seconds": pipe_s, "pipeline_gbp_s": round(gbp / pipe_s, 3), "database_load_seconds": load_s,
                      "busy_seconds_per_stage": stages,
@@ -151,7 +159,7 @@ def main():
                      "output_matches_oracle": bool(got1 == exp1 and got2 == exp2),
                      "kept_pairs_expected": int(keep.sum())})
         print(json.dumps(rows[-1]), file=sys.stderr)
-    print(json.dumps({"pairs": args.pairs, "threads": args.threads, "host_cores": os.cpu_count(), "gpus": args.gpus,
+    print(json.dumps({"pairs": args.pairs, "threads": thread_counts, "host_cores": os.cpu_count(), "gpus": args.gpus,
                       "table_cells": capacity, "db_save_seconds": round(t_save, 1), "oracle_seconds_all_cores": round(t_oracle, 1),
                       "note": "seconds = whole CLI process (CUDA context + database load + pipeline); stage_occupancy = busy seconds "
                               "of the stage summed over its threads / pipeline seconds (a value of 7 means seven threads' worth)",
