@@ -254,6 +254,35 @@ int nh_bgzf_compress(int device, const uint8_t *in, size_t n, uint8_t *out, size
  * mean over `iters` launches after one warm-up, in seconds. */
 int nh_bench_bgzf(int device, const uint8_t *in, size_t n, int iters, double *out_seconds);
 
+/* gzip decompression on the GPU: in[0..n) is a whole gzip file (one member or many, any deflate block types)
+ * and out gets what `gzip -dc` writes: bytes after the last member that do not start with 0x1f are ignored,
+ * as zlib's gzread ignores them.  NH_ERR_IO for a stream that is not gzip, corrupt or truncated (including a
+ * wrong CRC-32 or ISIZE and a distance too far back); NH_ERR_CAPACITY when out_cap is too small, with
+ * *out_len set to the size needed. */
+int nh_gunzip(int device, const uint8_t *in, size_t n, uint8_t *out, size_t out_cap, size_t *out_len);
+/* nh_gunzip with an explicit chunk and window size in compressed bytes (0: the defaults) and test flags;
+ * counts[NH_GUNZIP_NCOUNTS] (may be NULL) receives what ran, indexed by NH_GUNZIP_COUNT_*. */
+#define NH_GUNZIP_SHIFT_CANDIDATES 1 /* every other chunk's candidate start moved by one bit: forces repairs */
+#define NH_GUNZIP_COUNT_WINDOWS 0
+#define NH_GUNZIP_COUNT_CHUNKS 1
+#define NH_GUNZIP_COUNT_REPAIRED 2   /* chunks decoded again from their predecessor's stop */
+#define NH_GUNZIP_COUNT_OVERFLOWED 3 /* chunks whose output outgrew their slot */
+#define NH_GUNZIP_COUNT_MEMBERS 4
+#define NH_GUNZIP_COUNT_CARRIED 5    /* compressed bytes carried from one window into the next */
+/* device time, in nanoseconds (CUDA events), of each phase: finding block starts, the first decode of every
+ * chunk, repairs and spills, carrying the 32 KiB history through the chunks, resolving markers + CRC32 */
+#define NH_GUNZIP_COUNT_NS_FIND 6
+#define NH_GUNZIP_COUNT_NS_DECODE 7
+#define NH_GUNZIP_COUNT_NS_REDECODE 8
+#define NH_GUNZIP_COUNT_NS_WINDOW 9
+#define NH_GUNZIP_COUNT_NS_RESOLVE 10
+#define NH_GUNZIP_NCOUNTS 11
+int nh_debug_gunzip(int device, const uint8_t *in, size_t n, uint8_t *out, size_t out_cap, size_t *out_len,
+                    size_t chunk_bytes, size_t window_bytes, int flags, uint64_t *counts);
+/* Device time of nh_gunzip's kernels for in[0..n) (no copies of the input or the output): mean over `iters`
+ * runs after one warm-up, in seconds. */
+int nh_bench_gunzip(int device, const uint8_t *in, size_t n, int iters, double *out_seconds);
+
 /* Pinned host memory for callers that want true async copies. */
 void *nh_host_alloc(size_t bytes);
 void nh_host_free(void *p);

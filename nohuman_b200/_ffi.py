@@ -23,6 +23,11 @@ NH_ERR_UNSUPPORTED = -4
 NH_ERR_CAPACITY = -5
 NH_ERR_NOMEM = -6
 
+NH_GUNZIP_SHIFT_CANDIDATES = 1  # nh_debug_gunzip flag
+# nh_debug_gunzip counts[], in order
+GUNZIP_COUNTS = ("windows", "chunks", "repaired", "overflowed", "members", "carried",
+                 "ns_find", "ns_decode", "ns_redecode", "ns_window", "ns_resolve")
+
 
 class NhError(RuntimeError):
     def __init__(self, code: int, msg: str):
@@ -115,6 +120,10 @@ SYMBOLS = {
     "nh_last_batch_runs": (_i32, [_vp, _u64, _vp, _vp, _vp, _u64, C.POINTER(_u64)]),
     "nh_bgzf_compress": (_i32, [_i32, _vp, C.c_size_t, _vp, C.c_size_t, C.POINTER(C.c_size_t)]),
     "nh_bench_bgzf": (_i32, [_i32, _vp, C.c_size_t, _i32, C.POINTER(C.c_double)]),
+    "nh_gunzip": (_i32, [_i32, _vp, C.c_size_t, _vp, C.c_size_t, C.POINTER(C.c_size_t)]),
+    "nh_debug_gunzip": (_i32, [_i32, _vp, C.c_size_t, _vp, C.c_size_t, C.POINTER(C.c_size_t), C.c_size_t, C.c_size_t,
+                               _i32, C.POINTER(_u64)]),
+    "nh_bench_gunzip": (_i32, [_i32, _vp, C.c_size_t, _i32, C.POINTER(C.c_double)]),
     "nh_host_alloc": (_vp, [C.c_size_t]),
     "nh_host_free": (None, [_vp]),
     "nh_debug_minimizers": (_i32, [_vp, _vp, _vp, _u64, _vp, _vp, _vp]),

@@ -14,7 +14,8 @@ import ctypes as C
 import numpy as np
 
 from . import _ffi
-from ._ffi import BatchStats, DbInfo, Files, NhError, Params, RunStats, check, lib
+from ._ffi import (GUNZIP_COUNTS, NH_ERR_CAPACITY, BatchStats, DbInfo, Files, NhError, Params, RunStats, check,
+                   lib)
 
 
 def parse_confidence_score(text: str) -> float:
@@ -101,6 +102,38 @@ def bgzf_kernel_seconds(data: bytes, device: int = 0, iters: int = 10) -> float:
     """Device time of the BGZF kernels for `data` in one batch (nh_bench_bgzf), mean of `iters` launches."""
     t = C.c_double()
     check(lib().nh_bench_bgzf(int(device), data, len(data), int(iters), C.byref(t)))
+    return t.value
+
+
+def debug_gunzip(data: bytes, device: int = 0, chunk: int = 0, window: int = 0, flags: int = 0):
+    """(inflated bytes, counts) of the gzip stream `data` inflated on `device` with the given chunk and window
+    sizes in compressed bytes (0: the defaults) and nh_debug_gunzip flags; counts maps _ffi.GUNZIP_COUNTS to
+    what ran."""
+    n = len(data)
+    counts = (C.c_uint64 * len(GUNZIP_COUNTS))()
+    got = C.c_size_t()
+    cap = 4 * n + 65536  # FASTQ inflates about 4x; a larger stream is inflated again into the size it reported
+    for _ in range(2):
+        out = np.empty(cap, np.uint8)
+        rc = lib().nh_debug_gunzip(int(device), data, n, out.ctypes.data, cap, C.byref(got), int(chunk), int(window),
+                                   int(flags), counts)
+        if rc != NH_ERR_CAPACITY or got.value <= cap:
+            break
+        cap = got.value
+    check(rc)
+    return C.string_at(out.ctypes.data, got.value), dict(zip(GUNZIP_COUNTS, counts))
+
+
+def gunzip(data: bytes, device: int = 0) -> bytes:
+    """What `gzip -dc` gives for `data`, inflated on `device` (nh_gunzip): every member, trailing bytes that
+    do not start a member ignored.  NhError NH_ERR_IO for a corrupt or truncated stream."""
+    return debug_gunzip(data, device)[0]
+
+
+def gunzip_kernel_seconds(data: bytes, device: int = 0, iters: int = 3) -> float:
+    """Device time of nh_gunzip's kernels for the gzip stream `data` (nh_bench_gunzip), mean of `iters` runs."""
+    t = C.c_double()
+    check(lib().nh_bench_gunzip(int(device), data, len(data), int(iters), C.byref(t)))
     return t.value
 
 

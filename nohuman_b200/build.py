@@ -15,7 +15,7 @@ CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libnohuman_gpu.so")
 CLI = os.path.join(PKG, "bin", "nohuman")
 
-CU_SOURCES = ["nh_kernels.cu", "nh_capi.cu", "nh_synth.cu", "nh_deflate.cu"]
+CU_SOURCES = ["nh_kernels.cu", "nh_capi.cu", "nh_synth.cu", "nh_deflate.cu", "nh_inflate.cu"]
 CC_SOURCES = ["nh_pipeline.cc", "nh_pack.cc"]  # host pipeline and the host-side packer, compiled into the same library
 
 NVCC_FLAGS = [

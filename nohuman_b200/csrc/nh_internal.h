@@ -132,6 +132,61 @@ class GpuDeflater {
   uint64_t *d_offs_ = nullptr, *h_offs_ = nullptr;
 };
 
+/* nh_inflate.cu: gzip decompression on one GPU with its own stream, device buffers and pinned staging.
+ * inflate() reads the compressed stream from `src` a window at a time and hands the inflated bytes, in
+ * order, to `sink` — exactly the bytes zlib's gzread gives, or an error (NH_ERR_IO: truncated or corrupt).
+ * Not thread-safe: one per thread. */
+struct NhGzMember;
+struct NhGzChunk;
+struct NhGzEmit;
+struct NhGzJob;
+class GpuInflater {
+ public:
+  /* fills dst with up to `want` bytes; 0 at the end of the input, -1 on a read error */
+  typedef std::function<long(uint8_t *dst, size_t want)> Source;
+  /* receives the next run of inflated bytes; a nonzero return ends inflate() with that code */
+  typedef std::function<int(const uint8_t *, size_t)> Sink;
+  static constexpr size_t kChunkBytes = size_t(32) << 10;  /* compressed bytes per chunk */
+  static constexpr size_t kWindowBytes = size_t(16) << 20; /* new compressed bytes per window */
+  GpuInflater() = default;
+  GpuInflater(const GpuInflater &) = delete;
+  GpuInflater &operator=(const GpuInflater &) = delete;
+  ~GpuInflater();
+  /* NH_OK or an nh_status with nh_last_error() set; flags: NH_GUNZIP_SHIFT_CANDIDATES */
+  int open(int device, size_t chunk_bytes = 0, size_t window_bytes = 0, int flags = 0);
+  int inflate(const Source &src, const Sink &sink);
+  /* device time of the kernels for inflating in[0..n) (no input or output copies), mean of `iters` after one
+   * warm-up */
+  int time_kernels(const uint8_t *in, size_t n, int iters, double *seconds);
+  size_t device_bytes() const;
+  uint64_t counts[NH_GUNZIP_NCOUNTS] = {}; /* of the last inflate(): see nh_debug_gunzip */
+
+ private:
+  void lap(int a, int b, int count);
+  int device_ = -1, flags_ = 0;
+  size_t chunk_ = 0, window_ = 0, cap_ = 0;
+  uint32_t max_chunks_ = 0;
+  uint64_t slot_cap_ = 0, out_cap_ = 0, max_pieces_ = 0;
+  bool timing_ = false;
+  double kernel_s_ = 0;
+  cudaStream_t stream_ = nullptr;
+  cudaEvent_t ev_[8] = {};
+  uint8_t *d_win_[2] = {nullptr, nullptr}, *d_dicts_ = nullptr, *d_out_ = nullptr;
+  uint64_t *d_cand_ = nullptr, *d_piece_off_ = nullptr;
+  NhGzChunk *d_recs_ = nullptr;
+  uint16_t *d_slots_ = nullptr, *d_spill_ = nullptr;
+  NhGzMember *d_mrec_ = nullptr, *d_spill_mrec_ = nullptr;
+  NhGzEmit *d_emit_ = nullptr;
+  NhGzJob *d_jobs_ = nullptr, *h_jobs_ = nullptr;
+  uint32_t *d_piece_len_ = nullptr, *d_crcs_ = nullptr, *d_bad_ = nullptr;
+  uint8_t *h_in_ = nullptr, *h_out_ = nullptr;
+  NhGzChunk *h_recs_ = nullptr;
+  NhGzMember *h_mrec_ = nullptr;
+  NhGzEmit *h_emit_ = nullptr;
+  uint64_t *h_piece_off_ = nullptr;
+  uint32_t *h_piece_len_ = nullptr, *h_crcs_ = nullptr, *h_bad_ = nullptr;
+};
+
 int nh_set_error(int code, const char *fmt, ...);
 int nh_db_build_filter(nh_db *db); /* after the cells are on the device (every open path; the synthetic builder calls it itself) */
 /* zeroed table of `capacity` cells for the synthetic builder (nh_synth.cu), which fills it and builds the filter */
