@@ -40,7 +40,6 @@
 
 namespace {
 
-constexpr uint32_t BGZF_INPUT = 0xff00;   /* input bytes per member (bgzf_members) */
 constexpr uint32_t BGZF_SLOT = 65536;     /* device bytes reserved per member before compaction */
 constexpr int NT = 512;                   /* threads per member */
 constexpr int NSEG = 128;                 /* parse segments per member */
@@ -56,8 +55,8 @@ constexpr size_t SMEM_PREV = BGZF_INPUT * 2;         /* chain links (u16); later
 constexpr size_t SMEM_HEAD = (size_t(1) << HBITS) * 2; /* hash heads (u16); later the Huffman workspace */
 constexpr size_t SMEM_BYTES = SMEM_IN + SMEM_PREV + SMEM_HEAD;
 
-/* gzip member header up to the BC subfield's value: BGZF's fixed fields (bgzf_members) */
-__constant__ uint8_t c_gz_header[16] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0};
+/* gzip member header up to the BC subfield's value: BGZF's fixed fields (BGZF_HEADER) */
+__constant__ uint8_t c_gz_header[16] = {NH_BGZF_HEADER_BYTES};
 
 __constant__ uint8_t c_cl_order[19] = {16, 17, 18, 0, 8, 7, 9, 6, 10, 5, 11, 4, 12, 3, 13, 2, 14, 1, 15};
 

@@ -98,8 +98,17 @@ struct nh_session {
 void nh_pack_range(const uint8_t *bases, const uint64_t *offsets, uint64_t total_bases, uint64_t s0, uint64_t s1, uint8_t *codes,
                    uint32_t *valid, const uint32_t *poff);
 
+/* BGZF framing, shared by the zlib path (nh_pipeline.cc) and the GPU deflater (nh_deflate.cu), which must
+ * cut and frame members byte for byte alike.  Every member is a gzip member whose header carries one extra
+ * subfield, 'BC', holding the member's total size - 1 (the two bytes after these 16); output ends in
+ * bgzip's empty end-of-file member. */
+#define NH_BGZF_HEADER_BYTES 0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0
+constexpr uint32_t BGZF_INPUT = 0xff00; /* input bytes per member (the last member of a block may be shorter) */
+constexpr unsigned char BGZF_HEADER[16] = {NH_BGZF_HEADER_BYTES};
+constexpr unsigned char BGZF_EOF[28] = {NH_BGZF_HEADER_BYTES, 0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+
 /* nh_deflate.cu: BGZF compression on one GPU with its own stream, device buffers and pinned staging for a
- * batch of up to batch_bytes of input.  compress() cuts every block into 0xff00-byte members as the zlib
+ * batch of up to batch_bytes of input.  compress() cuts every block into BGZF_INPUT-byte members as the zlib
  * path does and returns each block's members, one string per block, or hands them in order to a sink; larger
  * inputs go in several rounds.
  * Not thread-safe: one per thread. */

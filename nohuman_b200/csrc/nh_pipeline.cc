@@ -46,7 +46,6 @@
 #include <deque>
 #include <algorithm>
 #include <atomic>
-#include <map>
 #include <memory>
 #include <unordered_map>
 #include <mutex>
@@ -56,6 +55,7 @@
 
 #include "../../include/nohuman_gpu.h"
 #include "nh_internal.h"
+#include "nh_ordered.h"
 
 extern char **environ;
 
@@ -147,12 +147,14 @@ static int spawn_filter(const std::vector<std::string> &argv, int stdin_fd, int 
  * compressed size in a 'BC' extra subfield, so members can be inflated in parallel */
 
 static bool bgzf_block_size(const unsigned char *hdr, size_t n, size_t *xlen, size_t *bsize) {
-  if (n < 12 || hdr[0] != 0x1f || hdr[1] != 0x8b || hdr[2] != 8 || !(hdr[3] & 4)) return false;
+  /* gzip magic and deflate (BGZF_HEADER[0..2]) with FEXTRA set */
+  if (n < 12 || memcmp(hdr, BGZF_HEADER, 3) != 0 || !(hdr[3] & 4)) return false;
   *xlen = hdr[10] | (size_t)hdr[11] << 8;
   if (n < 12 + *xlen) return false;
   for (size_t o = 12; o + 4 <= 12 + *xlen;) {
     const size_t slen = hdr[o + 2] | (size_t)hdr[o + 3] << 8;
-    if (hdr[o] == 'B' && hdr[o + 1] == 'C' && slen == 2 && o + 6 <= 12 + *xlen) {
+    /* 'B', 'C' and a 2-byte length: BGZF_HEADER[12..15] */
+    if (memcmp(hdr + o, BGZF_HEADER + 12, 4) == 0 && o + 6 <= 12 + *xlen) {
       *bsize = (hdr[o + 4] | (size_t)hdr[o + 5] << 8) + 1;
       return true;
     }
@@ -238,27 +240,17 @@ class BgzfReader {
   }
   /* next run of inflated bytes, in file order; 0 at the end, -1 on error */
   long next(std::string &out) {
-    std::shared_ptr<Blk> b;
-    {
-      std::unique_lock<std::mutex> lk(m_);
-      cv_.wait(lk, [&] { return (!order_.empty() && order_.front()->done) || (eof_ && order_.empty()) || error_; });
-      if (error_) return -1;
-      if (order_.empty()) return 0;
-      b = order_.front();
-      if (!b->ok) return -1;
-      order_.pop_front();
-      space_.notify_all();
+    std::shared_ptr<Blk> b = q_.pop();
+    if (!b) return failed_ ? -1 : 0;
+    if (!b->ok) {
+      fail();
+      return -1;
     }
     out.swap(b->raw);
     return (long)out.size();
   }
   void close() {
-    {
-      std::lock_guard<std::mutex> lk(m_);
-      stop_ = true;
-      cv_.notify_all();
-      space_.notify_all();
-    }
+    q_.stop();
     if (producer_.joinable()) producer_.join();
     for (auto &t : workers_)
       if (t.joinable()) t.join();
@@ -272,23 +264,13 @@ class BgzfReader {
   struct Blk {
     std::string comp, raw;
     std::vector<uint32_t> clen; /* deflate bytes + 8-byte trailer of each member in comp */
-    bool done = false, ok = true;
+    bool ok = true;
   };
-  bool enqueue(std::shared_ptr<Blk> b, bool inflated) {
-    std::unique_lock<std::mutex> lk(m_);
-    space_.wait(lk, [&] { return order_.size() < 64 || stop_; });
-    if (stop_) return false;
-    b->done = inflated;
-    order_.push_back(b);
-    if (!inflated) todo_.push_back(b);
-    cv_.notify_all();
-    return true;
-  }
+  typedef OrderedQueue<Blk> Queue;
+  /* a bad member or stream fails the whole reader at once: next() returns -1 from then on */
   void fail() {
-    std::lock_guard<std::mutex> lk(m_);
-    error_ = true;
-    eof_ = true;
-    cv_.notify_all();
+    failed_ = true;
+    q_.stop();
   }
   /* A member without the BC subfield (e.g. `cat blocked.gz plain.gz`): zlib and kraken2 read such a
    * file, so the rest of it is inflated as an ordinary gzip stream on this thread. */
@@ -306,11 +288,9 @@ class BgzfReader {
       if (n < 0) return fail();
       if (n == 0) break;
       b->raw.resize((size_t)n);
-      if (!enqueue(b, true)) return;
+      if (!q_.push(b, Queue::DONE)) return;
     }
-    std::lock_guard<std::mutex> lk(m_);
-    eof_ = true;
-    cv_.notify_all();
+    q_.close();
   }
   void produce() {
     bool at_end = false;
@@ -356,29 +336,16 @@ class BgzfReader {
         b->clen.push_back((uint32_t)len);
       }
       if (bad) return fail();
-      if (!b->clen.empty() && !enqueue(b, false)) return;
+      if (!b->clen.empty() && !q_.push(b, Queue::QUEUED)) return;
       if (plain_member) return serial_tail(hdr, n_hdr);
-      if (at_end) {
-        std::lock_guard<std::mutex> lk(m_);
-        eof_ = true;
-        cv_.notify_all();
-      }
     }
+    q_.close();
   }
   void work() {
     z_stream zs;
     memset(&zs, 0, sizeof zs);
     if (inflateInit2(&zs, -15) != Z_OK) return;
-    for (;;) {
-      std::shared_ptr<Blk> b;
-      {
-        std::unique_lock<std::mutex> lk(m_);
-        cv_.wait(lk, [&] { return !todo_.empty() || eof_ || stop_; });
-        if (stop_ || (todo_.empty() && eof_)) break;
-        if (todo_.empty()) continue;
-        b = todo_.front();
-        todo_.pop_front();
-      }
+    while (std::shared_ptr<Blk> b = q_.take()) {
       Busy busy(clk_, ST_INFLATE);
       bool ok = true;
       size_t total = 0, at = 0;
@@ -410,10 +377,8 @@ class BgzfReader {
         at += len;
       }
       std::string().swap(b->comp);
-      std::lock_guard<std::mutex> lk(m_);
       b->ok = ok;
-      b->done = true;
-      cv_.notify_all();
+      q_.done(b);
     }
     inflateEnd(&zs);
   }
@@ -421,10 +386,8 @@ class BgzfReader {
   StageClock *clk_ = nullptr;
   std::thread producer_;
   std::vector<std::thread> workers_;
-  std::mutex m_;
-  std::condition_variable cv_, space_;
-  std::deque<std::shared_ptr<Blk>> order_, todo_;
-  bool eof_ = false, error_ = false, stop_ = false;
+  Queue q_{64};
+  std::atomic<bool> failed_{false};
 };
 
 /* Decompressed bytes of one input file, produced ahead of the parser by a thread of its own
@@ -510,27 +473,14 @@ class InputStream {
   long next(std::string &out) {
     if (bgzf_) return bgzf_->next(out);
     std::string *b = nullptr;
-    {
-      std::unique_lock<std::mutex> lk(m_);
-      cv_.wait(lk, [&] { return !ready_.empty() || finished_; });
-      if (ready_.empty()) return failed_ ? -1 : 0;
-      b = ready_.front();
-      ready_.pop_front();
-    }
+    if (!ready_.pop(b)) return failed_ ? -1 : 0;
     out.swap(*b);
-    {
-      std::lock_guard<std::mutex> lk(m_);
-      free_.push_back(b);
-      cv_.notify_all();
-    }
+    free_.push(std::move(b));
     return (long)out.size();
   }
   void close() {
-    {
-      std::lock_guard<std::mutex> lk(m_);
-      stop_ = true;
-      cv_.notify_all();
-    }
+    ready_.close();
+    free_.close();
     if (producer_.joinable()) producer_.join();
     bgzf_.reset();
     if (file_) fclose(file_), file_ = nullptr;
@@ -548,18 +498,11 @@ class InputStream {
       if (!(WIFEXITED(st) && WEXITSTATUS(st) == 0)) child_failed_ = true;
     }
   }
+  /* fills the NBUF buffers in turn: a buffer goes back on free_ once next() has swapped its bytes out */
   void produce() {
-    for (int i = 0; i < NBUF; i++) free_.push_back(&bufs_[i]);
-    bool bad = false;
-    for (;;) {
-      std::string *b = nullptr;
-      {
-        std::unique_lock<std::mutex> lk(m_);
-        cv_.wait(lk, [&] { return !free_.empty() || stop_; });
-        if (stop_) break;
-        b = free_.front();
-        free_.pop_front();
-      }
+    for (int i = 0; i < NBUF; i++) free_.push(&bufs_[i]);
+    std::string *b = nullptr;
+    while (free_.pop(b)) {
       b->resize(BUF);
       long n;
       {
@@ -578,18 +521,13 @@ class InputStream {
         if (child_failed_) n = -1;
       }
       if (n <= 0) {
-        bad = n < 0;
+        failed_ = n < 0;
         break;
       }
       b->resize((size_t)n);
-      std::lock_guard<std::mutex> lk(m_);
-      ready_.push_back(b);
-      cv_.notify_all();
+      if (!ready_.push(std::move(b))) break;
     }
-    std::lock_guard<std::mutex> lk(m_);
-    failed_ = bad;
-    finished_ = true;
-    cv_.notify_all();
+    ready_.close();
   }
 
   std::unique_ptr<BgzfReader> bgzf_;
@@ -601,11 +539,9 @@ class InputStream {
   pid_t pid_ = -1;
   bool child_failed_ = false;
   std::thread producer_;
-  std::mutex m_;
-  std::condition_variable cv_;
   std::string bufs_[NBUF];
-  std::deque<std::string *> ready_, free_;
-  bool finished_ = false, failed_ = false, stop_ = false;
+  Channel<std::string *> ready_{NBUF}, free_{NBUF};
+  bool failed_ = false; /* set by the producer before it closes ready_ */
 };
 
 /* ------------------------------------------------------------------ */
@@ -890,10 +826,6 @@ struct ZstdLib {
  * compressed size in a 'BC' extra subfield.  Any gunzip reads it as ordinary multi-member gzip (which
  * is also what gzp writes for the reference, src/compression.rs:214-234); bgzip-aware tools and this
  * library's own reader can inflate the members in parallel. */
-static const size_t BGZF_INPUT = 0xff00;
-static const unsigned char BGZF_EOF[28] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0,
-                                           0x1b, 0, 3, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-
 static bool bgzf_members(const std::string &in, std::string &out) {
   z_stream zs;
   memset(&zs, 0, sizeof zs);
@@ -904,7 +836,7 @@ static bool bgzf_members(const std::string &in, std::string &out) {
   unsigned char buf[65536];
   bool ok = true;
   for (size_t pos = 0; pos < in.size() && ok; pos += BGZF_INPUT) {
-    const size_t n = std::min(BGZF_INPUT, in.size() - pos);
+    const size_t n = std::min<size_t>(BGZF_INPUT, in.size() - pos);
     deflateReset(&zs);
     zs.next_in = (Bytef *)in.data() + pos;
     zs.avail_in = (uInt)n;
@@ -915,9 +847,9 @@ static bool bgzf_members(const std::string &in, std::string &out) {
       break;
     }
     const size_t clen = zs.total_out, bsize = 18 + clen + 8;
-    const unsigned char hdr[18] = {0x1f, 0x8b, 8, 4, 0, 0, 0, 0, 0, 0xff, 6, 0, 'B', 'C', 2, 0,
-                                   (unsigned char)((bsize - 1) & 0xff), (unsigned char)((bsize - 1) >> 8)};
-    memcpy(buf, hdr, 18);
+    memcpy(buf, BGZF_HEADER, 16);
+    buf[16] = (unsigned char)((bsize - 1) & 0xff);
+    buf[17] = (unsigned char)((bsize - 1) >> 8);
     const uint32_t crc = (uint32_t)crc32(crc32(0L, Z_NULL, 0), (const Bytef *)in.data() + pos, (uInt)n);
     unsigned char *tr = buf + 18 + clen;
     for (int i = 0; i < 4; i++) tr[i] = (unsigned char)(crc >> (8 * i)), tr[4 + i] = (unsigned char)((uint32_t)n >> (8 * i));
@@ -1024,15 +956,16 @@ class OutputFile {
 struct Block {
   int file = 0;
   std::string raw, packed;
-  bool done = false;
+  bool ok = true;     /* false when compressing it failed */
+  int gpu_rc = NH_OK; /* a GPU deflater's failure and its message */
+  std::string gpu_msg;
 };
 
 /* Compresses blocks on `threads` host threads, or, given GPUs, on one deflater thread per GPU that takes
  * every waiting block up to GpuDeflater::kBatchBytes at a time; the flusher writes them in order. */
 class BlockWriter {
  public:
-  BlockWriter(OutputFile *files, int n_files, int threads, const std::vector<int> &gpus, StageClock *clk)
-      : files_(files), n_files_(n_files), clk_(clk) {
+  BlockWriter(OutputFile *files, int threads, const std::vector<int> &gpus, StageClock *clk) : files_(files), clk_(clk) {
     for (int dev : gpus) workers_.emplace_back([this, dev] { gpu_work(dev); });
     const int n = gpus.empty() ? (threads < 1 ? 1 : threads) : 0;
     for (int i = 0; i < n; i++) workers_.emplace_back([this] { work(); });
@@ -1043,49 +976,29 @@ class BlockWriter {
     auto b = std::make_shared<Block>();
     b->file = file;
     b->raw = std::move(raw);
-    std::unique_lock<std::mutex> lk(m_);
-    space_.wait(lk, [&] { return order_.size() < 64; });
-    order_.push_back(b);
-    if (files_[file].parallel())
-      todo_.push_back(b);
-    else
-      b->done = true;
-    cv_.notify_all();
+    q_.push(b, files_[file].parallel() ? Queue::QUEUED : Queue::DONE);
   }
   bool finish() {
-    {
-      std::lock_guard<std::mutex> lk(m_);
-      closing_ = true;
-      cv_.notify_all();
-    }
+    q_.close();
     for (auto &t : workers_) t.join();
     flusher_.join();
     return ok_;
   }
-  /* the first GPU deflater failure (NH_OK if none) and its message */
+  /* the first GPU deflater failure in output order (NH_OK if none) and its message */
   int error(std::string &msg) const {
     msg = err_msg_;
     return err_code_;
   }
 
  private:
+  typedef OrderedQueue<Block> Queue;
   void gpu_work(int device) {
     GpuDeflater gd;
     int rc = gd.open(device);
     std::string msg = rc ? nh_last_error() : "";
     for (;;) {
-      std::vector<std::shared_ptr<Block>> batch;
-      {
-        std::unique_lock<std::mutex> lk(m_);
-        cv_.wait(lk, [&] { return !todo_.empty() || closing_; });
-        if (todo_.empty()) return;
-        size_t bytes = 0;
-        while (!todo_.empty() && (batch.empty() || bytes + todo_.front()->raw.size() <= GpuDeflater::kBatchBytes)) {
-          bytes += todo_.front()->raw.size();
-          batch.push_back(todo_.front());
-          todo_.pop_front();
-        }
-      }
+      std::vector<std::shared_ptr<Block>> batch = q_.take(GpuDeflater::kBatchBytes, [](const Block &b) { return b.raw.size(); });
+      if (batch.empty()) return;
       if (rc == NH_OK) {
         Busy busy(clk_, ST_COMPRESS);
         std::vector<GpuDeflater::Span> spans;
@@ -1097,70 +1010,40 @@ class BlockWriter {
         else
           for (size_t i = 0; i < batch.size(); i++) batch[i]->packed = std::move(packed[i]);
       }
-      std::lock_guard<std::mutex> lk(m_);
-      if (rc != NH_OK) {
-        ok_ = false;
-        if (err_code_ == NH_OK) err_code_ = rc, err_msg_ = msg;
-      }
       for (auto &b : batch) {
+        if (rc != NH_OK) b->ok = false, b->gpu_rc = rc, b->gpu_msg = msg;
         b->raw.clear();
         b->raw.shrink_to_fit();
-        b->done = true;
       }
-      cv_.notify_all();
+      q_.done(batch);
     }
   }
   void work() {
-    for (;;) {
-      std::shared_ptr<Block> b;
-      {
-        std::unique_lock<std::mutex> lk(m_);
-        cv_.wait(lk, [&] { return !todo_.empty() || closing_; });
-        if (todo_.empty()) return;
-        b = todo_.front();
-        todo_.pop_front();
-      }
-      bool ok;
+    while (std::shared_ptr<Block> b = q_.take()) {
       {
         Busy busy(clk_, ST_COMPRESS);
-        ok = files_[b->file].compress_block(b->raw, b->packed);
+        b->ok = files_[b->file].compress_block(b->raw, b->packed);
       }
-      std::lock_guard<std::mutex> lk(m_);
-      if (!ok) ok_ = false;
       b->raw.clear();
       b->raw.shrink_to_fit();
-      b->done = true;
-      cv_.notify_all();
+      q_.done(b);
     }
   }
+  /* the only thread that writes ok_ and the error, so they need no lock */
   void flush() {
-    for (;;) {
-      std::shared_ptr<Block> b;
-      {
-        std::unique_lock<std::mutex> lk(m_);
-        cv_.wait(lk, [&] { return (!order_.empty() && order_.front()->done) || (closing_ && order_.empty()); });
-        if (order_.empty()) return;
-        b = order_.front();
-        order_.pop_front();
-        space_.notify_all();
-      }
+    while (std::shared_ptr<Block> b = q_.pop()) {
+      if (!b->ok) ok_ = false;
+      if (b->gpu_rc != NH_OK && err_code_ == NH_OK) err_code_ = b->gpu_rc, err_msg_ = b->gpu_msg;
       const std::string &s = files_[b->file].parallel() ? b->packed : b->raw;
       Busy busy(clk_, ST_WRITE);
-      if (!files_[b->file].write(s)) {
-        std::lock_guard<std::mutex> lk(m_);
-        ok_ = false;
-      }
+      if (!files_[b->file].write(s)) ok_ = false;
     }
   }
   OutputFile *files_;
-  int n_files_;
   StageClock *clk_;
-  std::mutex m_;
-  std::condition_variable cv_, space_;
-  std::deque<std::shared_ptr<Block>> order_, todo_;
+  Queue q_{64};
   std::vector<std::thread> workers_;
   std::thread flusher_;
-  bool closing_ = false;
   bool ok_ = true;
   int err_code_ = NH_OK;
   std::string err_msg_;
@@ -1170,7 +1053,6 @@ class BlockWriter {
 /* the pipeline                                                        */
 
 struct Work {
-  uint64_t id = 0;
   Chunk c[2];
   uint64_t n_units = 0;
   std::vector<uint32_t> call;
@@ -1190,6 +1072,42 @@ struct Decider {
   const uint8_t *fixed_keep = nullptr;
   const uint32_t *fixed_call = nullptr;
   uint64_t fixed_n = 0;
+};
+
+/* A classifier thread's GPU session and the pinned buffers it stages sub-batches in, freed with it. */
+struct GpuStaging {
+  nh_session *sess = nullptr;
+  uint8_t *h_bases = nullptr; /* cap_bases bases */
+  uint64_t *h_off = nullptr;  /* offsets of up to max_batch_seqs sequences, and the end */
+  uint64_t cap_bases = 0;
+  GpuStaging() = default;
+  GpuStaging(const GpuStaging &) = delete;
+  GpuStaging &operator=(const GpuStaging &) = delete;
+  ~GpuStaging() { release(); }
+  void release() {
+    if (sess) nh_session_destroy(sess), sess = nullptr;
+    if (h_bases) nh_host_free(h_bases), h_bases = nullptr;
+    if (h_off) nh_host_free(h_off), h_off = nullptr;
+    cap_bases = 0;
+  }
+  /* a session on `db` for sub-batches of up to `bases` bases and `seqs` sequences, made anew only when there
+   * is none yet or `bases` is more than the current one holds; "" or the reason it failed */
+  std::string fit(nh_db *db, nh_params_t p, uint64_t bases, size_t seqs) {
+    if (sess && bases <= cap_bases) return "";
+    release();
+    if (bases > (1ull << 31)) return "a single read (pair) of more than 2^31 bases is not supported";
+    p.max_batch_bases = bases;
+    p.max_batch_seqs = seqs;
+    h_bases = (uint8_t *)nh_host_alloc(bases);
+    h_off = (uint64_t *)nh_host_alloc(seqs * 8);
+    if (!h_bases || !h_off || nh_session_create(db, &p, &sess) != NH_OK) {
+      const std::string err = std::string("cannot set up a GPU session: ") + nh_last_error();
+      release();
+      return err;
+    }
+    cap_bases = bases;
+    return "";
+  }
 };
 
 static void append_record(std::string &out, const Chunk &c, const Rec &r, bool tagged, uint32_t ext) {
@@ -1378,7 +1296,6 @@ static int run_pipeline(const Decider &dec, const nh_files_t *files, nh_run_stat
   const int db_k = dec.dbs.empty() ? 0 : (int)dec.dbs[0]->info.k;
   const int db_amb_span = dec.dbs.empty() ? 0 : dec.dbs[0]->params.amb_span;
   const int threads = dec.params.threads < 1 ? 1 : dec.params.threads;
-  const bool keep_human = dec.params.keep_human != 0;
 
   std::string err;
   StageClock clock;
@@ -1427,38 +1344,31 @@ static int run_pipeline(const Decider &dec, const nh_files_t *files, nh_run_stat
       if (f == 0) cuts.close();
     });
 
-  /* classifiers */
-  std::mutex pair_m;
-  uint64_t next_id = 0;
+  /* classifiers: a Work enters `handoff` when it is taken and leaves to the writer in that order.
+   * Back-pressure: the GPU outruns the output compressor by orders of magnitude, so batches are only
+   * handed out while fewer than NH_MAX_AHEAD are inside. */
+  constexpr size_t NH_MAX_AHEAD = 8;
+  typedef OrderedQueue<Work> Handoff;
+  Handoff handoff(NH_MAX_AHEAD);
+  std::mutex pair_m; /* both files' chunks and the Work's place in `handoff` are taken as one step */
   bool input_done = false;
-  std::mutex done_m;
-  std::condition_variable done_cv;
-  std::map<uint64_t, std::unique_ptr<Work>> done;
-  bool failed = false;
-  std::string fail_msg;
-  int live_classifiers = 0;
-  /* back-pressure: the GPU outruns the output compressor by orders of magnitude, so batches
-   * are only handed out while fewer than NH_MAX_AHEAD are waiting for the writer */
-  constexpr uint64_t NH_MAX_AHEAD = 8;
-  std::mutex ahead_m;
-  std::condition_variable ahead_cv;
-  uint64_t written_id = 0;
 
-  auto take = [&]() -> std::unique_ptr<Work> {
+  auto take = [&]() -> std::shared_ptr<Work> {
     std::lock_guard<std::mutex> lk(pair_m);
     if (input_done) return nullptr;
-    {
-      std::unique_lock<std::mutex> al(ahead_m);
-      ahead_cv.wait(al, [&] { return next_id < written_id + NH_MAX_AHEAD; });
-    }
-    auto w = std::make_unique<Work>();
-    for (int f = 0; f < nf; f++) {
-      std::unique_ptr<Chunk> c;
-      if (!chunks[f].pop(c)) {
+    /* the Work enters before its chunks leave the readers' channels, so that a full window holds the
+     * chunks back in the channels; it enters empty if there turn out to be none */
+    auto w = std::make_shared<Work>();
+    if (!handoff.push(w, Handoff::CLAIMED)) return nullptr;
+    std::unique_ptr<Chunk> c[2];
+    for (int f = 0; f < nf; f++)
+      if (!chunks[f].pop(c[f])) {
         input_done = true;
+        handoff.done(w);
         return nullptr;
       }
-      w->c[f] = std::move(*c);
+    for (int f = 0; f < nf; f++) {
+      w->c[f] = std::move(*c[f]);
       if (!w->c[f].error.empty()) w->error = w->c[f].error;
       if (w->c[f].last) input_done = true;
     }
@@ -1468,7 +1378,6 @@ static int run_pipeline(const Decider &dec, const nh_files_t *files, nh_run_stat
       if (w->c[1].recs.size() < w->n_units) w->n_units = w->c[1].recs.size();
       input_done = true;
     }
-    w->id = next_id++;
     if (input_done) {
       for (int f = 0; f < nf; f++) chunks[f].close();
       cuts.close();
@@ -1480,19 +1389,15 @@ static int run_pipeline(const Decider &dec, const nh_files_t *files, nh_run_stat
    * up to four when -t allows it, because the same threads re-serialise the kept records */
   const int per_gpu = std::max(2, std::min(4, threads / 4));
   const int n_classifiers = dec.fixed_keep ? 1 : per_gpu * (int)dec.dbs.size();
-  live_classifiers = n_classifiers;
+  std::atomic<int> running_classifiers{n_classifiers};
+  nh_params_t sess_params = dec.params;
+  sess_params.emit_runs = want_lines ? 1 : 0;
   uint64_t fixed_cursor = 0;
   std::vector<std::thread> classifier_threads;
   for (int ci = 0; ci < n_classifiers; ci++)
     classifier_threads.emplace_back([&, ci] {
-      nh_session *sess = nullptr;
-      uint8_t *h_bases = nullptr;
-      uint64_t *h_off = nullptr;
-      size_t cap_bases = 0, cap_seqs = 0;
-      std::string my_err;
-      for (;;) {
-        std::unique_ptr<Work> w = take();
-        if (!w) break;
+      GpuStaging gpu;
+      while (std::shared_ptr<Work> w = take()) {
         if (w->error.empty() && w->n_units) {
           const uint64_t n_seqs = w->n_units * nf;
           uint64_t total = 0;
@@ -1518,30 +1423,8 @@ static int run_pipeline(const Decider &dec, const nh_files_t *files, nh_run_stat
               for (int f = 0; f < nf; f++) ub += w->c[f].recs[i].seq_len;
               longest = std::max(longest, ub);
             }
-            const uint64_t want_cap = std::max<uint64_t>(NH_BATCH_BASES, longest + 64);
-            if (!sess || want_cap > cap_bases) {
-              if (sess) nh_session_destroy(sess), sess = nullptr;
-              if (h_bases) nh_host_free(h_bases), h_bases = nullptr;
-              if (h_off) nh_host_free(h_off), h_off = nullptr;
-              cap_bases = (size_t)want_cap;
-              cap_seqs = (size_t)NH_CHUNK_RECORDS * nf + 2;
-              nh_params_t p = dec.params;
-              p.max_batch_bases = cap_bases;
-              p.max_batch_seqs = cap_seqs;
-              p.emit_runs = want_lines ? 1 : 0;
-              if (cap_bases > (1ull << 31))
-                w->error = "a single read (pair) of more than 2^31 bases is not supported";
-              else {
-                h_bases = (uint8_t *)nh_host_alloc(cap_bases);
-                h_off = (uint64_t *)nh_host_alloc(cap_seqs * 8);
-                if (!h_bases || !h_off || nh_session_create(dec.dbs[(size_t)ci % dec.dbs.size()], &p, &sess) != NH_OK) {
-                  w->error = std::string("cannot set up a GPU session: ") + nh_last_error();
-                  if (sess) nh_session_destroy(sess);
-                  sess = nullptr;
-                  cap_bases = 0;
-                }
-              }
-            }
+            w->error = gpu.fit(dec.dbs[(size_t)ci % dec.dbs.size()], sess_params,
+                               std::max<uint64_t>(NH_BATCH_BASES, longest + 64), (size_t)NH_CHUNK_RECORDS * nf + 2);
             if (want_lines && w->error.empty()) {
               w->first_run.assign(n_seqs + 1, 0);
               w->run_ext.resize(total + 1);
@@ -1555,23 +1438,23 @@ static int run_pipeline(const Decider &dec, const nh_files_t *files, nh_run_stat
               for (; u1 < w->n_units; u1++) {
                 uint64_t ub = 0;
                 for (int f = 0; f < nf; f++) ub += w->c[f].recs[u1].seq_len;
-                if (u1 > u0 && o + ub + 64 > cap_bases) break;
+                if (u1 > u0 && o + ub + 64 > gpu.cap_bases) break;
                 for (int f = 0; f < nf; f++) { /* mates interleaved: sequences 2i, 2i+1 */
                   const Rec &r = w->c[f].recs[u1];
-                  h_off[s++] = o;
-                  memcpy(h_bases + o, w->c[f].text.data() + r.seq_off, r.seq_len);
+                  gpu.h_off[s++] = o;
+                  memcpy(gpu.h_bases + o, w->c[f].text.data() + r.seq_off, r.seq_len);
                   o += r.seq_len;
                 }
               }
-              h_off[s] = o;
+              gpu.h_off[s] = o;
               }
               Busy classifying(&clock, ST_CLASSIFY);
-              if (nh_classify_batch(sess, h_bases, h_off, s, w->call.data() + u0, w->keep.data() + u0, nullptr) != NH_OK)
+              if (nh_classify_batch(gpu.sess, gpu.h_bases, gpu.h_off, s, w->call.data() + u0, w->keep.data() + u0, nullptr) != NH_OK)
                 w->error = std::string("classification failed: ") + nh_last_error();
               if (want_lines && w->error.empty()) {
                 uint64_t nr = 0;
                 uint32_t *fr = w->first_run.data() + u0 * nf;
-                if (nh_last_batch_runs(sess, s, fr, w->run_ext.data() + runs_at, w->run_len.data() + runs_at,
+                if (nh_last_batch_runs(gpu.sess, s, fr, w->run_ext.data() + runs_at, w->run_len.data() + runs_at,
                                        total + 1 - runs_at, &nr) != NH_OK)
                   w->error = std::string("reading the hit runs failed: ") + nh_last_error();
                 else {
@@ -1611,43 +1494,23 @@ static int run_pipeline(const Decider &dec, const nh_files_t *files, nh_run_stat
             if (!want_report) std::vector<Rec>().swap(w->c[f].recs);
           }
         }
-        std::lock_guard<std::mutex> lk(done_m);
-        done[w->id] = std::move(w);
-        done_cv.notify_all();
+        handoff.done(w);
       }
-      if (sess) nh_session_destroy(sess);
-      if (h_bases) nh_host_free(h_bases);
-      if (h_off) nh_host_free(h_off);
-      std::lock_guard<std::mutex> lk(done_m);
-      live_classifiers--;
-      done_cv.notify_all();
+      if (--running_classifiers == 0) handoff.close(); /* no Work will enter any more */
     });
 
-  /* writer (this thread): batches in id order; gzip output is deflated on the sessions' GPUs on request */
+  /* writer (this thread): batches in input order; gzip output is deflated on the sessions' GPUs on request */
   std::vector<int> deflate_gpus;
   if (dec.params.gpu_gzip && fmt == 'g')
     for (const nh_db *db : dec.dbs)
       if (std::find(deflate_gpus.begin(), deflate_gpus.end(), db->info.device) == deflate_gpus.end())
         deflate_gpus.push_back(db->info.device);
-  BlockWriter bw(outs, nf, threads, deflate_gpus, &clock);
-  uint64_t want = 0, total_units = 0, n_classified = 0, total_bases = 0;
+  BlockWriter bw(outs, threads, deflate_gpus, &clock);
+  uint64_t total_units = 0, n_classified = 0, total_bases = 0;
+  bool failed = false;
+  std::string fail_msg;
   std::string pend[2];
-  for (;;) {
-    std::unique_ptr<Work> w;
-    {
-      std::unique_lock<std::mutex> lk(done_m);
-      done_cv.wait(lk, [&] { return done.count(want) || live_classifiers == 0; });
-      auto it = done.find(want);
-      if (it == done.end()) break;
-      w = std::move(it->second);
-      done.erase(it);
-    }
-    want++;
-    {
-      std::lock_guard<std::mutex> al(ahead_m);
-      written_id = want;
-      ahead_cv.notify_all();
-    }
+  while (std::shared_ptr<Work> w = handoff.pop()) {
     if (!w->error.empty()) {
       if (!failed) fail_msg = w->error;
       failed = true;
@@ -1685,7 +1548,6 @@ static int run_pipeline(const Decider &dec, const nh_files_t *files, nh_run_stat
   for (auto &t : reader_threads) t.join();
   bool wrote = bw.finish();
   for (int f = 0; f < nf; f++) wrote = outs[f].close() && wrote;
-  (void)keep_human;
   if (kout) {
     const bool closed_ok = fclose(kout) == 0;
     kout = nullptr;

@@ -70,7 +70,9 @@ def read_output(path, fmt):
     raw = open(path, "rb").read()
     if fmt == "g":
         assert raw[:2] == b"\x1f\x8b"
-        return gzip.decompress(raw)  # handles concatenated members
+        # gzip -dc reads concatenated members in one pass; gzip.decompress copies the rest of the input once per
+        # member, which takes minutes on outputs of thousands of members
+        return subprocess.run(["gzip", "-dc", str(path)], check=True, capture_output=True).stdout
     if fmt == "b":
         assert raw[:3] == b"BZh"
         return bz2.decompress(raw)
@@ -103,18 +105,24 @@ def read_output(path, fmt):
     return raw
 
 
-@pytest.mark.parametrize("fmt", ["u", "g", "b", "x", "z"])
-def test_single_end_formats(tmp_path, fmt):
+@pytest.mark.parametrize("fmt,n,threads", [
+    *(pytest.param(fmt, 5000, 3, id=fmt) for fmt in ["u", "g", "b", "x", "z"]),
+    # one compressor thread keeps the writer behind the classifier.  The writer stalls once the block writer
+    # holds 64 blocks of 1 MiB (about 5 batches of 65536 records at half of them kept); the 19 batches here
+    # are enough for 8 more to wait in the hand-off, so its window fills and must still keep the order
+    pytest.param("g", 1_200_000, 1, id="g-slow-writer"),
+])
+def test_single_end_formats(tmp_path, fmt, n, threads):
     if fmt == "b" and not shutil.which("bzip2") or fmt == "x" and not shutil.which("xz"):
         pytest.skip("compressor CLI missing")
-    recs = make_records(5000, seed=1)
+    recs = make_records(n, seed=1)
     rng = np.random.default_rng(2)
     keep = rng.integers(0, 2, size=len(recs), dtype=np.uint8)
     call = np.where(keep == 0, 9606, 0).astype(np.uint32)  # default mode: kept == unclassified
     inp, out = tmp_path / "in.fq", tmp_path / f"out.{fmt}"
     write_input(inp, recs)
-    st = rewrite_files(keep, call, inp, out, out_format=fmt, threads=3)
-    assert (st.total, st.classified, st.unclassified) == (5000, int((call != 0).sum()), int((call == 0).sum()))
+    st = rewrite_files(keep, call, inp, out, out_format=fmt, threads=threads)
+    assert (st.total, st.classified, st.unclassified) == (n, int((call != 0).sum()), int((call == 0).sum()))
     assert st.bases == sum(len(s) for _, s, _ in recs)
     assert read_output(out, fmt) == expected(recs, keep, call)
 
@@ -218,16 +226,26 @@ def test_unusual_but_valid_endings(tmp_path):
 def test_gzip_output_is_bgzf_and_is_read_back_in_parallel(tmp_path):
     """gzip output = BGZF (members <= 64 KiB with a 'BC' size subfield + bgzip's EOF marker); such input
     (bgzip, bcl2fastq, our own output) is inflated by several threads and must give identical records"""
+    check_bgzf_round_trip(tmp_path, 30000, write_threads=4)
+
+
+def test_bgzf_round_trip_fills_the_reader_and_writer_windows(tmp_path):
+    """The same with more than 64 MiB per file: the writer holds at most 64 blocks of 1 MiB and the parallel
+    reader at most 64 tasks of 16 members, so both windows fill up and must still keep the order."""
+    n = 170_000  # about 73 MB of FASTQ per file: more than 64 x 16 members, more than 64 blocks
+    check_bgzf_round_trip(tmp_path, n, write_threads=8, min_members=64 * 16)
+
+
+def check_bgzf_round_trip(tmp_path, n, write_threads, min_members=50):
     import struct
     import zlib
-    n = 30000
     r1, r2 = make_records(n, seed=11), make_records(n, seed=12)
     keep, call = np.ones(n, np.uint8), np.zeros(n, np.uint32)
     i1, i2 = tmp_path / "p_1.fq", tmp_path / "p_2.fq"
     write_input(i1, r1)
     write_input(i2, r2)
     g1, g2 = tmp_path / "g_1.fq.gz", tmp_path / "g_2.fq.gz"
-    rewrite_files(keep, call, i1, g1, i2, g2, out_format="g", threads=4)
+    rewrite_files(keep, call, i1, g1, i2, g2, out_format="g", threads=write_threads)
     raw = open(g1, "rb").read()
     assert raw[:4] == b"\x1f\x8b\x08\x04" and raw[12:16] == b"BC\x02\x00"
     assert raw.endswith(bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000"))
@@ -241,8 +259,8 @@ def test_gzip_output_is_bgzf_and_is_read_back_in_parallel(tmp_path):
         total += isize
         members += 1
         pos += bsize
-    assert pos == len(raw) and members > 50 and total == len(expected(r1, keep, call))
-    assert gzip.decompress(raw) == expected(r1, keep, call)
+    assert pos == len(raw) and members > min_members and total == len(expected(r1, keep, call))
+    assert read_output(g1, "g") == expected(r1, keep, call)
     assert subprocess.run(["gzip", "-t", str(g1)]).returncode == 0
     # read it back with 8 threads (parallel member inflate) and with 1 (zlib's gzread): same bytes
     for threads in (8, 1):
