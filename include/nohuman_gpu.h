@@ -283,6 +283,56 @@ int nh_debug_gunzip(int device, const uint8_t *in, size_t n, uint8_t *out, size_
  * runs after one warm-up, in seconds. */
 int nh_bench_gunzip(int device, const uint8_t *in, size_t n, int iters, double *out_seconds);
 
+/* ---- database build: kraken2-build --build on the GPU ----
+ * nh_build_taxonomy converts an NCBI taxonomy dump to taxo.k2d (host only, no GPU).  Every taxid that
+ * seqid2taxid assigns is marked with all its ancestors; the marked nodes are numbered breadth-first from
+ * taxid 1 (internal id 1, so every parent id is below its children's), with the children of a node taken in
+ * ascending external taxid (a choice made so that the image is deterministic); node 0 is the zeroed
+ * "unclassified" node.  Names are the `scientific name` rows of names.dmp, ranks column 3 of nodes.dmp.
+ * NH_ERR_IO with the file and line in nh_last_error() for a map taxid missing from nodes.dmp, a parent
+ * cycle, a node that does not reach taxid 1, or a malformed line.  *node_count (may be NULL) includes node 0. */
+int nh_build_taxonomy(const char *nodes_dmp, const char *names_dmp, const char *seqid2taxid, const char *out_taxo_k2d,
+                      uint64_t *node_count);
+
+typedef struct {
+  const char *const *fasta; /* library files: FASTA, plain / gzip / bzip2 */
+  int32_t n_fasta;
+  const char *nodes_dmp, *names_dmp, *seqid2taxid;
+  const char *out_dir;      /* receives hash.k2d, opts.k2d, taxo.k2d (created if missing) */
+  uint32_t k, l, spaces;    /* 0: kraken2-build's defaults 35 / 31 / 7 */
+  uint64_t capacity;        /* table cells; 0: estimated from the library (an extra pass over it) */
+  double load_factor;       /* of the estimated capacity; 0: 0.7 */
+  uint64_t batch_bases;     /* bases per device batch; 0: 256 MiB.  Longer sequences are cut into pieces */
+  int32_t threads;          /* host threads for reading blocked gzip (BGZF) input; <= 0: 1 */
+  int32_t device;
+} nh_build_params_t;
+
+typedef struct {
+  uint64_t sequences;  /* library records inserted */
+  uint64_t skipped;    /* records whose ID has no seqid2taxid entry (kraken2 warns and skips them too) */
+  uint64_t bases;      /* bases of the inserted records */
+  uint64_t minimizers; /* minimizer insertions (runs of equal consecutive non-ambiguous minimizers count once) */
+  uint64_t estimate;   /* distinct minimizers estimated by the capacity pass (0 when capacity was given) */
+  uint64_t estimate_slots;   /* size of the capacity pass's device set of sampled hashes when it ended */
+  uint64_t estimate_rescans; /* batches the capacity pass scanned again after they overfilled the set */
+  uint64_t capacity, size, node_count; /* of the written table / taxonomy */
+  double s_taxonomy, s_estimate, s_insert, s_write; /* wall seconds per phase */
+} nh_build_stats_t;
+
+/* Builds a kraken2 database from FASTA files and an NCBI taxonomy, as `kraken2-build --build` does for a
+ * nucleotide library.  A record's ID is the first word of its header, looked up in seqid2taxid; records
+ * without an entry are skipped and counted.  Bases other than ACGT / acgt are ambiguous (N, and dustmasker's
+ * x).  Every non-ambiguous minimizer is inserted with CompactHashTable::CompareAndSet and the LCA merge on
+ * the GPU.  Every lookup on the result returns what a sequential build returns for the same library, except
+ * where two distinct minimizers share a compacted key on one probe path (kraken2 merges those by design, and
+ * which one survives depends on insertion order): the cell layout is NOT byte-reproducible between runs, as
+ * with any concurrent CompareAndSet build.  The files are written as *.tmp and renamed only once all three
+ * are complete; if a rename fails, the ones already renamed are removed, so a failed build leaves none of its
+ * .k2d files behind (a file of an earlier build in out_dir that a completed rename replaced is gone too).
+ * NH_ERR_CAPACITY ("table full") once the load passes 0.95: the inserts stop soon after, the overshoot being at
+ * most the claims of the tiles already running (up to 256 cells per running warp).  stats may be NULL. */
+int nh_build_db(const nh_build_params_t *p, nh_build_stats_t *stats);
+
 /* Pinned host memory for callers that want true async copies. */
 void *nh_host_alloc(size_t bytes);
 void nh_host_free(void *p);

@@ -90,6 +90,29 @@ class Files(C.Structure):
     ]
 
 
+class BuildParams(C.Structure):
+    _fields_ = [
+        ("fasta", C.POINTER(C.c_char_p)), ("n_fasta", C.c_int32),
+        ("nodes_dmp", C.c_char_p), ("names_dmp", C.c_char_p), ("seqid2taxid", C.c_char_p),
+        ("out_dir", C.c_char_p),
+        ("k", C.c_uint32), ("l", C.c_uint32), ("spaces", C.c_uint32),
+        ("capacity", C.c_uint64), ("load_factor", C.c_double), ("batch_bases", C.c_uint64),
+        ("threads", C.c_int32), ("device", C.c_int32),
+    ]
+
+
+class BuildStats(C.Structure):
+    _fields_ = [
+        ("sequences", C.c_uint64), ("skipped", C.c_uint64), ("bases", C.c_uint64), ("minimizers", C.c_uint64),
+        ("estimate", C.c_uint64), ("estimate_slots", C.c_uint64), ("estimate_rescans", C.c_uint64),
+        ("capacity", C.c_uint64), ("size", C.c_uint64), ("node_count", C.c_uint64),
+        ("s_taxonomy", C.c_double), ("s_estimate", C.c_double), ("s_insert", C.c_double), ("s_write", C.c_double),
+    ]
+
+    def as_dict(self):
+        return {f: getattr(self, f) for f, _ in self._fields_}
+
+
 # every symbol include/nohuman_gpu.h declares: name -> (restype, argtypes)
 _vp, _u64, _i32 = C.c_void_p, C.c_uint64, C.c_int
 SYMBOLS = {
@@ -124,6 +147,8 @@ SYMBOLS = {
     "nh_debug_gunzip": (_i32, [_i32, _vp, C.c_size_t, _vp, C.c_size_t, C.POINTER(C.c_size_t), C.c_size_t, C.c_size_t,
                                _i32, C.POINTER(_u64)]),
     "nh_bench_gunzip": (_i32, [_i32, _vp, C.c_size_t, _i32, C.POINTER(C.c_double)]),
+    "nh_build_taxonomy": (_i32, [C.c_char_p, C.c_char_p, C.c_char_p, C.c_char_p, C.POINTER(_u64)]),
+    "nh_build_db": (_i32, [C.POINTER(BuildParams), C.POINTER(BuildStats)]),
     "nh_host_alloc": (_vp, [C.c_size_t]),
     "nh_host_free": (None, [_vp]),
     "nh_debug_minimizers": (_i32, [_vp, _vp, _vp, _u64, _vp, _vp, _vp]),

@@ -10,12 +10,13 @@ computation happens in libnohuman_gpu.so (CUDA, sm_100a).
 from __future__ import annotations
 
 import ctypes as C
+import os
 
 import numpy as np
 
 from . import _ffi
-from ._ffi import (GUNZIP_COUNTS, NH_ERR_CAPACITY, BatchStats, DbInfo, Files, NhError, Params, RunStats, check,
-                   lib)
+from ._ffi import (GUNZIP_COUNTS, NH_ERR_CAPACITY, BatchStats, BuildParams, BuildStats, DbInfo, Files, NhError, Params,
+                   RunStats, check, lib)
 
 
 def parse_confidence_score(text: str) -> float:
@@ -135,6 +136,36 @@ def gunzip_kernel_seconds(data: bytes, device: int = 0, iters: int = 3) -> float
     t = C.c_double()
     check(lib().nh_bench_gunzip(int(device), data, len(data), int(iters), C.byref(t)))
     return t.value
+
+
+def build_taxonomy(nodes_dmp, names_dmp, seqid2taxid, out_taxo_k2d) -> int:
+    """taxo.k2d from an NCBI taxonomy dump, for the taxids seqid2taxid assigns and their ancestors
+    (nh_build_taxonomy; host only).  Returns the node count, node 0 included."""
+    n = C.c_uint64()
+    check(lib().nh_build_taxonomy(str(nodes_dmp).encode(), str(names_dmp).encode(), str(seqid2taxid).encode(),
+                                  str(out_taxo_k2d).encode(), C.byref(n)))
+    return int(n.value)
+
+
+def build_db(fasta, nodes_dmp, names_dmp, seqid2taxid, out_dir, k: int = 35, l: int = 31, spaces: int = 7,
+             capacity: int = 0, load_factor: float = 0.7, threads: int = os.cpu_count() or 1, device: int = 0,
+             batch_bases: int = 0) -> BuildStats:
+    """kraken2-build --build on `device` (nh_build_db): hash.k2d / opts.k2d / taxo.k2d into out_dir from the FASTA
+    files `fasta` (a path or a list; plain, gzip or bzip2) and an NCBI taxonomy.  capacity 0 estimates it from
+    the library; batch_bases 0 takes the default batch size."""
+    files = [fasta] if isinstance(fasta, (str, os.PathLike)) else list(fasta)
+    arr = (C.c_char_p * max(len(files), 1))(*[str(f).encode() for f in files])
+    p = BuildParams()
+    p.fasta = C.cast(arr, C.POINTER(C.c_char_p))
+    p.n_fasta = len(files)
+    p.nodes_dmp, p.names_dmp = str(nodes_dmp).encode(), str(names_dmp).encode()
+    p.seqid2taxid, p.out_dir = str(seqid2taxid).encode(), str(out_dir).encode()
+    p.k, p.l, p.spaces = int(k), int(l), int(spaces)
+    p.capacity, p.load_factor, p.batch_bases = int(capacity), float(load_factor), int(batch_bases)
+    p.threads, p.device = int(threads), int(device)
+    st = BuildStats()
+    check(lib().nh_build_db(C.byref(p), C.byref(st)))
+    return st
 
 
 class Database:
@@ -378,4 +409,5 @@ class Session:
         self.close()
 
 
-__all__ = ["Database", "Session", "NhError", "BatchStats", "DbInfo", "parse_confidence_score"]
+__all__ = ["Database", "Session", "NhError", "BatchStats", "BuildStats", "DbInfo", "build_db", "build_taxonomy",
+           "parse_confidence_score"]

@@ -196,6 +196,24 @@ class GpuInflater {
   uint32_t *h_piece_len_ = nullptr, *h_crcs_ = nullptr, *h_bad_ = nullptr;
 };
 
+/* nh_pipeline.cc: the records of one FASTA or FASTQ file (plain, gzip, BGZF with `threads` inflaters, bzip2),
+ * read by the file pipeline's reader; inflating runs ahead on a thread of its own. */
+class NhSeqReader {
+ public:
+  NhSeqReader();
+  NhSeqReader(const NhSeqReader &) = delete;
+  NhSeqReader &operator=(const NhSeqReader &) = delete;
+  ~NhSeqReader();
+  int open(const char *path, int threads); /* NH_OK, or NH_ERR_IO with nh_last_error() set */
+  /* The next record: its header line (with the '>') and its sequence lines joined, valid until the next call.
+   * 1: a record, 0: end of file, NH_ERR_IO: a read error (truncated or corrupt input) or malformed record. */
+  int next(const char **hdr, size_t *hdr_len, const char **seq, size_t *seq_len);
+
+ private:
+  struct Impl;
+  Impl *impl_;
+};
+
 int nh_set_error(int code, const char *fmt, ...);
 int nh_db_build_filter(nh_db *db); /* after the cells are on the device (every open path; the synthetic builder calls it itself) */
 /* zeroed table of `capacity` cells for the synthetic builder (nh_synth.cu), which fills it and builds the filter */

@@ -1621,3 +1621,41 @@ extern "C" int nh_debug_rewrite_files(const nh_files_t *files, const uint8_t *ke
   d.fixed_n = n_units;
   return run_pipeline(d, files, stats);
 }
+
+/* ------------------------------------------------------------------ */
+/* NhSeqReader: the reader above, a record at a time (nh_build.cu)     */
+
+struct NhSeqReader::Impl {
+  RecordReader reader;
+  Chunk chunk;
+  size_t next = 0;
+};
+
+NhSeqReader::NhSeqReader() : impl_(new Impl()) {}
+NhSeqReader::~NhSeqReader() { delete impl_; }
+
+int NhSeqReader::open(const char *path, int threads) {
+  std::string err;
+  if (!impl_->reader.open(path, threads < 1 ? 1 : threads, err, nullptr)) return nh_set_error(NH_ERR_IO, "%s", err.c_str());
+  return NH_OK;
+}
+
+int NhSeqReader::next(const char **hdr, size_t *hdr_len, const char **seq, size_t *seq_len) {
+  Impl &m = *impl_;
+  while (m.next >= m.chunk.recs.size()) {
+    if (m.chunk.last) return 0;
+    m.reader.next_chunk(m.chunk);
+    m.next = 0;
+    if (!m.chunk.error.empty()) {
+      m.chunk.recs.clear();
+      m.chunk.last = true;
+      return nh_set_error(NH_ERR_IO, "%s", m.chunk.error.c_str());
+    }
+  }
+  const Rec &r = m.chunk.recs[m.next++];
+  *hdr = m.chunk.text.data() + r.hdr_off;
+  *hdr_len = r.hdr_len;
+  *seq = m.chunk.text.data() + r.seq_off;
+  *seq_len = r.seq_len;
+  return 1;
+}

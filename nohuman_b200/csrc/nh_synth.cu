@@ -13,6 +13,7 @@
 
 #include "../../include/nohuman_synth.h"
 #include "nh_internal.h"
+#include "nh_insert.cuh"
 #include "nh_kernels.cuh"
 
 #define CUDA_TRY(expr)                                                                       \
@@ -41,76 +42,19 @@ k_synth_genome(uint8_t *__restrict__ out, uint64_t start, uint64_t n, uint64_t s
 }
 
 /* ------------------------------------------------------------------ */
-/* build: CompareAndSet loop of build_db.cc collapsed to value := LCA(old, taxon) */
+/* build: the genome is cut into blocks of block_bases, block i belongs to leaf i mod n_leaves, and the last
+ * overlap_frac of every block belongs to the next block's leaf too, so that LCA values appear in the table */
 
-__device__ __forceinline__ uint32_t d_lca(const uint32_t *parent, uint32_t a, uint32_t b) {
-  if (!a || !b) return a ? a : b;
-  while (a != b) {
-    if (a > b)
-      a = parent[a];
-    else
-      b = parent[b];
-  }
-  return a;
-}
-
-/* returns 1 if a previously empty cell was claimed */
-__device__ uint32_t cht_insert_lca(const NhDbParams &db, uint32_t *cells, uint64_t key,
-                                   uint32_t taxon) {
-  const uint64_t h = nh_fmix64(key);
-  if (db.min_hash && h < db.min_hash) return 0;
-  const uint32_t ckey = (uint32_t)(h >> (32u + db.value_bits));
-  uint64_t idx = nh_fastmod(h, db.capacity, db.mod_m, db.mod_sh1, db.mod_sh2);
-  for (uint64_t probes = 0; probes < db.capacity;) {
-    uint32_t cell = *((volatile uint32_t *)&cells[idx]);
-    if ((cell & db.value_mask) == 0u) {
-      const uint32_t want = (ckey << db.value_bits) | taxon;
-      const uint32_t old = atomicCAS(&cells[idx], 0u, want);
-      if (old == 0u) return 1;
-      cell = old; /* somebody else claimed it: examine what they wrote */
-    }
-    if ((cell >> db.value_bits) == ckey) {
-      for (;;) {
-        const uint32_t cur = cell & db.value_mask;
-        const uint32_t nv = d_lca(db.parent, cur, taxon);
-        if (nv == cur) return 0;
-        const uint32_t want = (ckey << db.value_bits) | nv;
-        const uint32_t old = atomicCAS(&cells[idx], cell, want);
-        if (old == cell) return 0;
-        cell = old;
-      }
-    }
-    idx++;
-    if (idx >= db.capacity) idx = 0;
-    probes++;
-  }
-  return 0; /* table full: caller sees the load factor stall */
-}
-
-__global__ void __launch_bounds__(NH_BLOCK_THREADS)
-k_insert_tiles(const NhDbParams db, uint32_t *cells, const NhBatchPtrs b, uint64_t chunk_start,
-               const uint32_t *__restrict__ leaf_taxa, uint32_t n_leaves, uint64_t block_bases,
-               uint64_t overlap_start, unsigned long long *size_counter) {
-  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
-  const uint32_t n_tiles = b.counters->n_tiles;
-  uint32_t claimed = 0;
-  for (uint32_t tile = blockIdx.x * NH_WARPS_PER_BLOCK + warp; tile < n_tiles;
-       tile += gridDim.x * NH_WARPS_PER_BLOCK) {
-    const NhTile t = b.tiles[tile];
-    const NhTileOut to = b.tile_out[tile];
+struct BlockTaxa {
+  const uint32_t *leaf_taxa;
+  uint32_t n_leaves;
+  uint64_t chunk_start, block_bases, overlap_start;
+  __device__ uint2 operator()(const NhTile &t) const {
     const uint64_t g = chunk_start + t.pos_begin;
     const uint64_t blk = g / block_bases, r = g % block_bases;
-    const uint32_t ta = leaf_taxa[blk % n_leaves];
-    const uint32_t tb = r >= overlap_start ? leaf_taxa[(blk + 1) % n_leaves] : 0u;
-    for (uint32_t j = lane; j < to.lk_cnt; j += 32u) {
-      const uint64_t key = b.lk_min[to.lk_off + j];
-      claimed += cht_insert_lca(db, cells, key, ta);
-      if (tb) claimed += cht_insert_lca(db, cells, key, tb);
-    }
+    return make_uint2(leaf_taxa[blk % n_leaves], r >= overlap_start ? leaf_taxa[(blk + 1) % n_leaves] : 0u);
   }
-  claimed = __reduce_add_sync(0xFFFFFFFFu, claimed);
-  if (lane == 0 && claimed) atomicAdd(size_counter, (unsigned long long)claimed);
-}
+};
 
 extern "C" int nh_synth_build_db(const void *opts, size_t opts_len, const void *taxo,
                                  size_t taxo_len, const uint32_t *leaf_taxa, int n_leaves,
@@ -146,9 +90,9 @@ extern "C" int nh_synth_build_db(const void *opts, size_t opts_len, const void *
   uint32_t *d_leaf = nullptr;
   unsigned long long *d_size = nullptr;
   cudaError_t e = cudaMalloc(&d_leaf, n_leaves * 4);
-  if (e == cudaSuccess) e = cudaMalloc(&d_size, 8);
+  if (e == cudaSuccess) e = cudaMalloc(&d_size, 16); /* claimed cells, and the full flag k_insert_tiles never sets here */
   if (e == cudaSuccess) e = cudaMemcpy(d_leaf, leaf_taxa, n_leaves * 4, cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMemset(d_size, 0, 8);
+  if (e == cudaSuccess) e = cudaMemset(d_size, 0, 16);
   const uint64_t target = (uint64_t)(p->target_load * (double)p->capacity);
   const uint64_t overlap_start =
       (uint64_t)((1.0 - (p->overlap_frac < 0 ? 0 : p->overlap_frac)) * (double)p->block_bases);
@@ -184,9 +128,8 @@ extern "C" int nh_synth_build_db(const void *opts, size_t opts_len, const void *
     B.counters = s->d_counters;
     nh_launch_plan(db->params, B, st);
     nh_launch_minimizers(db->params, B, (uint32_t)(n / (uint64_t)db->params.tile_pos + 2), sm, st);
-    k_insert_tiles<<<sm * 8, NH_BLOCK_THREADS, 0, st>>>(db->params, db->d_cells, B, gpos, d_leaf,
-                                                        (uint32_t)n_leaves, p->block_bases,
-                                                        overlap_start, d_size);
+    const BlockTaxa taxa{d_leaf, (uint32_t)n_leaves, gpos, p->block_bases, overlap_start};
+    k_insert_tiles<<<sm * 8, NH_BLOCK_THREADS, 0, st>>>(db->params, db->d_cells, B, taxa, ~0ull, d_size);
     unsigned long long prev = size;
     e = cudaMemcpyAsync(&size, d_size, 8, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);

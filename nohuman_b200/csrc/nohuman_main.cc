@@ -365,6 +365,175 @@ static int kraken2_shim(int argc, char **argv) {
 }
 
 /* ------------------------------------------------------------------ */
+/* invoked as `kraken2-build`: --build over kraken2-build's directory   */
+/* layout (DIR/taxonomy, DIR/library, DIR/seqid2taxid.map)              */
+
+static bool has_suffix(const std::string &s, const char *suf) {
+  const size_t n = strlen(suf);
+  return s.size() >= n && s.compare(s.size() - n, n, suf) == 0;
+}
+
+/* every regular file under dir, recursively, in name order */
+static void walk_files(const std::string &dir, std::vector<std::string> &out) {
+  DIR *d = opendir(dir.c_str());
+  if (!d) return;
+  std::vector<std::string> names;
+  while (dirent *e = readdir(d))
+    if (strcmp(e->d_name, ".") && strcmp(e->d_name, "..")) names.push_back(e->d_name);
+  closedir(d);
+  std::sort(names.begin(), names.end());
+  for (auto &n : names) {
+    const std::string p = path_join(dir, n);
+    if (is_dir(p))
+      walk_files(p, out);
+    else
+      out.push_back(p);
+  }
+}
+
+static bool is_library_file(const std::string &p) {
+  std::string f = path_file_name(p);
+  for (const char *z : {".gz", ".bz2"})
+    if (has_suffix(f, z)) f.resize(f.size() - strlen(z));
+  return has_suffix(f, ".fna") || has_suffix(f, ".fa") || has_suffix(f, ".fasta");
+}
+
+/* seqid2taxid.map from the TAXID lines of the prelim_map*.txt files anywhere under DIR/library, as kraken2-build's
+ * wrapper writes it */
+static bool write_seqid2taxid(const std::vector<std::string> &files, const std::string &out, std::string &err) {
+  std::string map;
+  size_t n_prelim = 0;
+  for (auto &p : files) {
+    const std::string f = path_file_name(p);
+    if (f.rfind("prelim_map", 0) != 0 || !has_suffix(f, ".txt")) continue;
+    n_prelim++;
+    FILE *in = fopen(p.c_str(), "r");
+    if (!in) {
+      err = "cannot open " + p;
+      return false;
+    }
+    char *line = nullptr;
+    size_t cap = 0;
+    ssize_t len;
+    int ln = 0;
+    while ((len = getline(&line, &cap, in)) >= 0) {
+      ln++;
+      std::string s(line, (size_t)len);
+      while (!s.empty() && (s.back() == '\n' || s.back() == '\r')) s.pop_back();
+      if (s.empty()) continue;
+      const size_t t1 = s.find('\t'), t2 = t1 == std::string::npos ? t1 : s.find('\t', t1 + 1);
+      const std::string kind = s.substr(0, t1);
+      if (kind == "TAXID" && t2 != std::string::npos) {
+        map += s.substr(t1 + 1, t2 - t1 - 1) + "\t" + s.substr(t2 + 1) + "\n";
+        continue;
+      }
+      err = p + ":" + std::to_string(ln) +
+            (kind == "ACCNUM" ? ": ACCNUM lines need accession2taxid lookups, which this build does not do; "
+                                "give the library a seqid2taxid.map"
+                              : ": malformed prelim_map line (expected TAXID<tab>sequence ID<tab>taxid)");
+      free(line);
+      fclose(in);
+      return false;
+    }
+    free(line);
+    fclose(in);
+  }
+  if (!n_prelim) {
+    err = "no seqid2taxid.map and no library/**/prelim_map*.txt to make it from";
+    return false;
+  }
+  FILE *o = fopen(out.c_str(), "w");
+  bool ok = o && fwrite(map.data(), 1, map.size(), o) == map.size();
+  if (o && fclose(o) != 0) ok = false;
+  if (!ok) err = "cannot write " + out;
+  return ok;
+}
+
+static int kraken2_build_shim(int argc, char **argv) {
+  static option opts[] = {{"build", 0, 0, 'b'},           {"db", 1, 0, 'd'},
+                          {"threads", 1, 0, 't'},         {"kmer-len", 1, 0, 'k'},
+                          {"minimizer-len", 1, 0, 'l'},   {"minimizer-spaces", 1, 0, 's'},
+                          {"load-factor", 1, 0, 'f'},     {"gpu", 1, 0, 'g'},
+                          {"download-taxonomy", 0, 0, 1}, {"download-library", 1, 0, 2},
+                          {"add-to-library", 1, 0, 3},    {"standard", 0, 0, 4},
+                          {"special", 1, 0, 5},           {"clean", 0, 0, 6},
+                          {0, 0, 0, 0}};
+  static const char *why[] = {"",
+                              "--download-taxonomy is not supported: it needs the network; put nodes.dmp and names.dmp in DIR/taxonomy",
+                              "--download-library is not supported: it needs the network; put FASTA files in DIR/library",
+                              "--add-to-library is not supported: it masks low-complexity regions with dustmasker; copy "
+                              "(masked) FASTA files into DIR/library and give DIR/seqid2taxid.map",
+                              "--standard is not supported: it downloads the standard libraries over the network",
+                              "--special is not supported: it downloads the special databases over the network",
+                              "--clean is not supported: remove DIR/library and DIR/taxonomy yourself"};
+  bool build = false;
+  std::string db;
+  int threads = 1, gpu = 0;
+  unsigned k = 35, l = 31, s = 7;
+  double lf = 0.7;
+  int c;
+  while ((c = getopt_long(argc, argv, "", opts, nullptr)) != -1) switch (c) {
+      case 'b': build = true; break;
+      case 'd': db = optarg; break;
+      case 't': threads = atoi(optarg); break;
+      case 'k': k = (unsigned)atoi(optarg); break;
+      case 'l': l = (unsigned)atoi(optarg); break;
+      case 's': s = (unsigned)atoi(optarg); break;
+      case 'f': lf = strtod(optarg, nullptr); break;
+      case 'g': gpu = atoi(optarg); break;
+      case 1: case 2: case 3: case 4: case 5: case 6:
+        fprintf(stderr, "kraken2-build (GPU): %s\n", why[c]);
+        return 64;
+      default: return 64;
+    }
+  if (!build || db.empty()) {
+    fprintf(stderr, "kraken2-build (GPU): only --build --db DIR is supported\n");
+    return 64;
+  }
+  const std::string lib_dir = path_join(db, "library"), tax_dir = path_join(db, "taxonomy");
+  std::vector<std::string> all, fasta;
+  walk_files(lib_dir, all);
+  for (auto &p : all)
+    if (is_library_file(p)) fasta.push_back(p);
+  if (fasta.empty()) return fail("no *.fna / *.fa / *.fasta (optionally .gz / .bz2) under %s", lib_dir.c_str());
+  const std::string map = path_join(db, "seqid2taxid.map");
+  if (!exists(map)) {
+    std::string err;
+    if (!write_seqid2taxid(all, map, err)) return fail("%s", err.c_str());
+    logmsg("INFO", "wrote %s from the library's prelim_map files", map.c_str());
+  }
+  std::vector<const char *> fp;
+  for (auto &p : fasta) fp.push_back(p.c_str());
+  const std::string nodes = path_join(tax_dir, "nodes.dmp"), names = path_join(tax_dir, "names.dmp");
+  nh_build_params_t p;
+  memset(&p, 0, sizeof p);
+  p.fasta = fp.data();
+  p.n_fasta = (int32_t)fp.size();
+  p.nodes_dmp = nodes.c_str();
+  p.names_dmp = names.c_str();
+  p.seqid2taxid = map.c_str();
+  p.out_dir = db.c_str();
+  p.k = k;
+  p.l = l;
+  p.spaces = s;
+  p.load_factor = lf;
+  p.threads = threads;
+  p.device = gpu;
+  nh_build_stats_t st;
+  if (nh_build_db(&p, &st)) return fail("kraken2-build: %s", nh_last_error());
+  fprintf(stderr, "Taxonomy: %llu nodes (%.3f s)\n", (unsigned long long)st.node_count, st.s_taxonomy);
+  if (st.estimate)
+    fprintf(stderr, "Estimated %llu distinct minimizers, capacity %llu (%.3f s)\n", (unsigned long long)st.estimate,
+            (unsigned long long)st.capacity, st.s_estimate);
+  fprintf(stderr, "Inserted %llu sequences (%.2f Mbp, %llu minimizers; %llu skipped without a seqid2taxid entry) (%.3f s)\n",
+          (unsigned long long)st.sequences, st.bases / 1e6, (unsigned long long)st.minimizers,
+          (unsigned long long)st.skipped, st.s_insert);
+  fprintf(stderr, "Wrote hash.k2d (capacity %llu, size %llu), opts.k2d, taxo.k2d to %s (%.3f s)\n",
+          (unsigned long long)st.capacity, (unsigned long long)st.size, db.c_str(), st.s_write);
+  return 0;
+}
+
+/* ------------------------------------------------------------------ */
 
 static void usage() {
   puts("Remove human reads from a sequencing run (B200 build of nohuman's kraken2 path)\n\n"
@@ -392,6 +561,7 @@ static void usage() {
 
 int main(int argc, char **argv) {
   if (path_file_name(argv[0]) == "kraken2") return kraken2_shim(argc, argv);
+  if (path_file_name(argv[0]) == "kraken2-build") return kraken2_build_shim(argc, argv);
   static option opts[] = {{"out1", 1, 0, 'o'},         {"out2", 1, 0, 'O'},          {"check", 0, 0, 'c'},
                           {"download", 0, 0, 'd'},     {"db", 1, 0, 'D'},            {"db-version", 1, 0, 1},
                           {"list-db-versions", 0, 0, 2}, {"output-type", 1, 0, 'F'}, {"threads", 1, 0, 't'},
