@@ -333,6 +333,43 @@ typedef struct {
  * most the claims of the tiles already running (up to 256 cells per running warp).  stats may be NULL. */
 int nh_build_db(const nh_build_params_t *p, nh_build_stats_t *stats);
 
+/* ---- low-complexity masking: dustmasker's symmetric DUST on the GPU ----
+ * The mask (DESIGN.md §4f): over every run of A/C/G/T in either case (every other byte ends a run), the union
+ * of the bases of every "perfect" triplet interval that fits in `window` bases, at score threshold `level`.
+ * window 4..64 and level 1..255 (dustmasker's defaults: 64, 20); anything else is NH_ERR_INVALID.
+ * nh_dust_mask: records concatenated in host memory, offsets[n_seqs+1] (offsets[0] = 0); out[i] is seq[i]
+ * lower-cased where masked and upper-cased everywhere else, which is dustmasker's FASTA form. */
+int nh_dust_mask(int device, const uint8_t *seq, const uint64_t *offsets, uint64_t n_seqs, int window, int level,
+                 uint8_t *out);
+
+#define NH_DUST_FASTA 0    /* dustmasker -outfmt fasta: headers as read, masked bases lower-case, 60 a line */
+#define NH_DUST_INTERVAL 1 /* dustmasker -outfmt interval: each header, then "start - end" lines, 0-based inclusive */
+typedef struct {
+  const char *in_path;  /* FASTA (or FASTQ): plain, gzip, BGZF or bzip2 */
+  const char *out_path; /* NULL or "-": stdout */
+  int32_t format;       /* NH_DUST_FASTA or NH_DUST_INTERVAL */
+  int32_t window;       /* 0: 64 */
+  int32_t level;        /* 0: 20 */
+  int32_t threads;      /* host threads for reading blocked gzip (BGZF) input; <= 0: 1 */
+  int32_t device;
+  uint64_t batch_bases; /* bases per device batch, 8192..2^31; 0: 256 MiB.  Longer records are cut into pieces */
+} nh_dust_params_t;
+
+typedef struct {
+  uint64_t sequences, bases, masked; /* records, their bases, masked bases */
+  uint64_t intervals;                /* maximal runs of masked bases */
+  double seconds;                    /* wall clock */
+} nh_dust_stats_t;
+
+/* File to file: every record of in_path masked and written as dustmasker writes it.  Headers are copied byte
+ * for byte.  An unreadable, corrupt or truncated input is NH_ERR_IO, and a failed run removes out_path.
+ * stats may be NULL. */
+int nh_dust_fasta(const nh_dust_params_t *p, nh_dust_stats_t *stats);
+/* Device time of nh_dust_mask's kernels at window 64, level 20 for records already on the device: mean over
+ * `iters` runs after one warm-up, in seconds. */
+int nh_bench_dust(int device, const uint8_t *seq, const uint64_t *offsets, uint64_t n_seqs, int iters,
+                  double *out_seconds);
+
 /* Pinned host memory for callers that want true async copies. */
 void *nh_host_alloc(size_t bytes);
 void nh_host_free(void *p);

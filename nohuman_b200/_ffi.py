@@ -113,6 +113,27 @@ class BuildStats(C.Structure):
         return {f: getattr(self, f) for f, _ in self._fields_}
 
 
+NH_DUST_FASTA = 0
+NH_DUST_INTERVAL = 1
+
+
+class DustParams(C.Structure):
+    _fields_ = [
+        ("in_path", C.c_char_p), ("out_path", C.c_char_p), ("format", C.c_int32), ("window", C.c_int32),
+        ("level", C.c_int32), ("threads", C.c_int32), ("device", C.c_int32), ("batch_bases", C.c_uint64),
+    ]
+
+
+class DustStats(C.Structure):
+    _fields_ = [
+        ("sequences", C.c_uint64), ("bases", C.c_uint64), ("masked", C.c_uint64), ("intervals", C.c_uint64),
+        ("seconds", C.c_double),
+    ]
+
+    def as_dict(self):
+        return {f: getattr(self, f) for f, _ in self._fields_}
+
+
 # every symbol include/nohuman_gpu.h declares: name -> (restype, argtypes)
 _vp, _u64, _i32 = C.c_void_p, C.c_uint64, C.c_int
 SYMBOLS = {
@@ -149,6 +170,9 @@ SYMBOLS = {
     "nh_bench_gunzip": (_i32, [_i32, _vp, C.c_size_t, _i32, C.POINTER(C.c_double)]),
     "nh_build_taxonomy": (_i32, [C.c_char_p, C.c_char_p, C.c_char_p, C.c_char_p, C.POINTER(_u64)]),
     "nh_build_db": (_i32, [C.POINTER(BuildParams), C.POINTER(BuildStats)]),
+    "nh_dust_mask": (_i32, [_i32, _vp, _vp, _u64, _i32, _i32, _vp]),
+    "nh_dust_fasta": (_i32, [C.POINTER(DustParams), C.POINTER(DustStats)]),
+    "nh_bench_dust": (_i32, [_i32, _vp, _vp, _u64, _i32, C.POINTER(C.c_double)]),
     "nh_host_alloc": (_vp, [C.c_size_t]),
     "nh_host_free": (None, [_vp]),
     "nh_debug_minimizers": (_i32, [_vp, _vp, _vp, _u64, _vp, _vp, _vp]),

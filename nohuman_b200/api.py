@@ -15,8 +15,8 @@ import os
 import numpy as np
 
 from . import _ffi
-from ._ffi import (GUNZIP_COUNTS, NH_ERR_CAPACITY, BatchStats, BuildParams, BuildStats, DbInfo, Files, NhError, Params,
-                   RunStats, check, lib)
+from ._ffi import (GUNZIP_COUNTS, NH_DUST_FASTA, NH_DUST_INTERVAL, NH_ERR_CAPACITY, BatchStats, BuildParams, BuildStats,
+                   DbInfo, DustParams, DustStats, Files, NhError, Params, RunStats, check, lib)
 
 
 def parse_confidence_score(text: str) -> float:
@@ -166,6 +166,50 @@ def build_db(fasta, nodes_dmp, names_dmp, seqid2taxid, out_dir, k: int = 35, l: 
     st = BuildStats()
     check(lib().nh_build_db(C.byref(p), C.byref(st)))
     return st
+
+
+def _records(seqs):
+    seqs = [s.encode() if isinstance(s, str) else bytes(s) for s in seqs]
+    offsets = np.zeros(len(seqs) + 1, np.uint64)
+    np.cumsum([len(s) for s in seqs], out=offsets[1:])
+    return seqs, b"".join(seqs), offsets
+
+
+def dust_mask(seqs, window: int = 64, level: int = 20, device: int = 0) -> list[bytes]:
+    """dustmasker's symmetric DUST on `device` (nh_dust_mask): each sequence (bytes or str) comes back with its
+    masked bases lower-cased and every other byte upper-cased."""
+    seqs, data, offsets = _records(seqs)
+    out = np.empty(max(len(data), 1), np.uint8)
+    check(lib().nh_dust_mask(int(device), data, offsets.ctypes.data, len(seqs), int(window), int(level),
+                             out.ctypes.data))
+    out = out[:len(data)].tobytes()
+    return [out[int(offsets[i]):int(offsets[i + 1])] for i in range(len(seqs))]
+
+
+def dust_fasta(in_path, out_path, fmt: str = "fasta", window: int = 64, level: int = 20,
+               threads: int = os.cpu_count() or 1, device: int = 0, batch_bases: int = 0) -> DustStats:
+    """`dustmasker -in in_path -out out_path -outfmt fmt` on `device` (nh_dust_fasta): fmt "fasta" (masked
+    bases lower-case) or "interval"; out_path None or "-" writes to stdout.  A failed run removes out_path."""
+    if fmt not in ("fasta", "interval"):
+        raise ValueError(f"unknown DUST output format {fmt!r} (fasta or interval)")
+    p = DustParams()
+    p.in_path = str(in_path).encode()
+    p.out_path = None if out_path is None else str(out_path).encode()
+    p.format = NH_DUST_FASTA if fmt == "fasta" else NH_DUST_INTERVAL
+    p.window, p.level, p.threads, p.device, p.batch_bases = int(window), int(level), int(threads), int(device), \
+        int(batch_bases)
+    st = DustStats()
+    check(lib().nh_dust_fasta(C.byref(p), C.byref(st)))
+    return st
+
+
+def dust_kernel_seconds(seqs, device: int = 0, iters: int = 5) -> float:
+    """Device time of nh_dust_mask's kernels (window 64, level 20) over `seqs` (nh_bench_dust), mean of
+    `iters` runs."""
+    seqs, data, offsets = _records(seqs)
+    t = C.c_double()
+    check(lib().nh_bench_dust(int(device), data, offsets.ctypes.data, len(seqs), int(iters), C.byref(t)))
+    return t.value
 
 
 class Database:
@@ -409,5 +453,5 @@ class Session:
         self.close()
 
 
-__all__ = ["Database", "Session", "NhError", "BatchStats", "BuildStats", "DbInfo", "build_db", "build_taxonomy",
-           "parse_confidence_score"]
+__all__ = ["Database", "Session", "NhError", "BatchStats", "BuildStats", "DbInfo", "DustStats", "build_db",
+           "build_taxonomy", "dust_fasta", "dust_kernel_seconds", "dust_mask", "parse_confidence_score"]

@@ -15,7 +15,7 @@ CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libnohuman_gpu.so")
 CLI = os.path.join(PKG, "bin", "nohuman")
 
-CU_SOURCES = ["nh_kernels.cu", "nh_capi.cu", "nh_synth.cu", "nh_deflate.cu", "nh_inflate.cu", "nh_build.cu"]
+CU_SOURCES = ["nh_kernels.cu", "nh_capi.cu", "nh_synth.cu", "nh_deflate.cu", "nh_inflate.cu", "nh_build.cu", "nh_dust.cu"]
 CC_SOURCES = ["nh_pipeline.cc", "nh_pack.cc"]  # host pipeline and the host-side packer, compiled into the same library
 
 NVCC_FLAGS = [
@@ -70,9 +70,9 @@ def build(force: bool = False, verbose: bool = False) -> str:
         cmd = ["/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++", "-O2", "-std=c++17", "-Wall",
                "-o", CLI, main_cc, "-L", PKG, "-lnohuman_gpu", "-Wl,-rpath,$ORIGIN/..", "-lpthread"]
         subprocess.check_call(cmd)
-        # the same binary under the names nohuman looks for on $PATH (src/main.rs:170) and the one that builds
-        # a database for it: argv shims
-        for name in ("kraken2", "kraken2-build"):
+        # the same binary under the names nohuman looks for on $PATH (src/main.rs:170), the one that builds
+        # a database for it and the masker kraken2-build --add-to-library runs: argv shims
+        for name in ("kraken2", "kraken2-build", "dustmasker"):
             shim = os.path.join(os.path.dirname(CLI), name)
             if os.path.lexists(shim):
                 os.remove(shim)

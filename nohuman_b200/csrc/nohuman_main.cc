@@ -461,8 +461,9 @@ static int kraken2_build_shim(int argc, char **argv) {
   static const char *why[] = {"",
                               "--download-taxonomy is not supported: it needs the network; put nodes.dmp and names.dmp in DIR/taxonomy",
                               "--download-library is not supported: it needs the network; put FASTA files in DIR/library",
-                              "--add-to-library is not supported: it masks low-complexity regions with dustmasker; copy "
-                              "(masked) FASTA files into DIR/library and give DIR/seqid2taxid.map",
+                              "--add-to-library is not supported: mask with \"dustmasker -in F -outfmt fasta | sed -e "
+                              "'/^>/!s/[a-z]/x/g'\" (nohuman_b200/bin/dustmasker runs on the GPU) into DIR/library and "
+                              "give DIR/seqid2taxid.map",
                               "--standard is not supported: it downloads the standard libraries over the network",
                               "--special is not supported: it downloads the special databases over the network",
                               "--clean is not supported: remove DIR/library and DIR/taxonomy yourself"};
@@ -533,6 +534,59 @@ static int kraken2_build_shim(int argc, char **argv) {
   return 0;
 }
 
+/* dustmasker -in F [-out F] [-outfmt fasta|interval] [-window N] [-level N]: what kraken2-build's
+ * mask_low_complexity.sh passes, run by nh_dust_fasta.  Any other option is refused with one line. */
+static int dustmasker_shim(int argc, char **argv) {
+  std::string in, out, fmt = "interval";
+  int window = 64, level = 20;
+  for (int i = 1; i < argc; i++) {
+    const std::string o = argv[i];
+    if (o != "-in" && o != "-out" && o != "-outfmt" && o != "-window" && o != "-level") {
+      fprintf(stderr, "dustmasker (GPU): option %s is not supported (only -in, -out, -outfmt, -window, -level)\n", o.c_str());
+      return 64;
+    }
+    if (i + 1 >= argc) {
+      fprintf(stderr, "dustmasker (GPU): option %s needs a value\n", o.c_str());
+      return 64;
+    }
+    const char *v = argv[++i];
+    if (o == "-in") in = v;
+    if (o == "-out") out = v;
+    if (o == "-outfmt") fmt = v;
+    if (o == "-window" || o == "-level") {
+      char *end = nullptr;
+      const long x = strtol(v, &end, 10);
+      const long lo = o == "-window" ? 4 : 1, hi = o == "-window" ? 64 : 255;
+      if (!*v || *end || x < lo || x > hi) {
+        fprintf(stderr, "dustmasker (GPU): %s %s is out of range (%ld..%ld)\n", o.c_str(), v, lo, hi);
+        return 64;
+      }
+      (o == "-window" ? window : level) = (int)x;
+    }
+  }
+  if (fmt != "fasta" && fmt != "interval") {
+    fprintf(stderr, "dustmasker (GPU): -outfmt %s is not supported (fasta or interval)\n", fmt.c_str());
+    return 64;
+  }
+  if (in.empty()) {
+    fprintf(stderr, "dustmasker (GPU): -in FILE is required\n");
+    return 64;
+  }
+  nh_dust_params_t p;
+  memset(&p, 0, sizeof p);
+  p.in_path = in.c_str();
+  p.out_path = out.empty() ? nullptr : out.c_str();
+  p.format = fmt == "fasta" ? NH_DUST_FASTA : NH_DUST_INTERVAL;
+  p.window = window;
+  p.level = level;
+  p.threads = 4;
+  if (nh_dust_fasta(&p, nullptr)) {
+    fprintf(stderr, "dustmasker (GPU): %s\n", nh_last_error());
+    return 1;
+  }
+  return 0;
+}
+
 /* ------------------------------------------------------------------ */
 
 static void usage() {
@@ -562,6 +616,7 @@ static void usage() {
 int main(int argc, char **argv) {
   if (path_file_name(argv[0]) == "kraken2") return kraken2_shim(argc, argv);
   if (path_file_name(argv[0]) == "kraken2-build") return kraken2_build_shim(argc, argv);
+  if (path_file_name(argv[0]) == "dustmasker") return dustmasker_shim(argc, argv);
   static option opts[] = {{"out1", 1, 0, 'o'},         {"out2", 1, 0, 'O'},          {"check", 0, 0, 'c'},
                           {"download", 0, 0, 'd'},     {"db", 1, 0, 'D'},            {"db-version", 1, 0, 1},
                           {"list-db-versions", 0, 0, 2}, {"output-type", 1, 0, 'F'}, {"threads", 1, 0, 't'},
