@@ -370,6 +370,20 @@ int nh_dust_fasta(const nh_dust_params_t *p, nh_dust_stats_t *stats);
 int nh_bench_dust(int device, const uint8_t *seq, const uint64_t *offsets, uint64_t n_seqs, int iters,
                   double *out_seconds);
 
+/* ---- database inspection: kraken2-inspect on the GPU ----
+ * Minimizers stored per internal taxon id in the resident table, as kraken2's GetValueCounts counts them.
+ * counts[n_counts] with n_counts >= node_count.  Cells whose value is not a taxo.k2d node (>= node_count) are
+ * counted in *out_of_range and not in counts.  *occupied counts every cell with a non-zero value. */
+int nh_db_taxon_counts(const nh_db *db, uint64_t *counts, uint64_t n_counts, uint64_t *occupied,
+                       uint64_t *out_of_range);
+#define NH_INSPECT_SKIP_COUNTS 1 /* header lines only (--skip-counts) */
+#define NH_INSPECT_ZERO_COUNTS 2 /* every node, zero counts too (--report-zero-counts) */
+/* kraken2-inspect's output for an open database; out_path NULL or "-": stdout.  NH_ERR_IO, and nothing is
+ * written, when some cell's value is not a taxo.k2d node or the occupied cells differ from the header's size. */
+int nh_db_inspect(const nh_db *db, const char *out_path, int32_t flags);
+/* Device time of k_taxon_counts over the resident table: mean over `iters` launches after one warm-up. */
+int nh_bench_taxon_counts(const nh_db *db, int iters, double *out_seconds);
+
 /* Pinned host memory for callers that want true async copies. */
 void *nh_host_alloc(size_t bytes);
 void nh_host_free(void *p);

@@ -116,6 +116,9 @@ class BuildStats(C.Structure):
 NH_DUST_FASTA = 0
 NH_DUST_INTERVAL = 1
 
+NH_INSPECT_SKIP_COUNTS = 1  # nh_db_inspect flags
+NH_INSPECT_ZERO_COUNTS = 2
+
 
 class DustParams(C.Structure):
     _fields_ = [
@@ -173,6 +176,9 @@ SYMBOLS = {
     "nh_dust_mask": (_i32, [_i32, _vp, _vp, _u64, _i32, _i32, _vp]),
     "nh_dust_fasta": (_i32, [C.POINTER(DustParams), C.POINTER(DustStats)]),
     "nh_bench_dust": (_i32, [_i32, _vp, _vp, _u64, _i32, C.POINTER(C.c_double)]),
+    "nh_db_taxon_counts": (_i32, [_vp, _vp, _u64, C.POINTER(_u64), C.POINTER(_u64)]),
+    "nh_db_inspect": (_i32, [_vp, C.c_char_p, C.c_int32]),
+    "nh_bench_taxon_counts": (_i32, [_vp, _i32, C.POINTER(C.c_double)]),
     "nh_host_alloc": (_vp, [C.c_size_t]),
     "nh_host_free": (None, [_vp]),
     "nh_debug_minimizers": (_i32, [_vp, _vp, _vp, _u64, _vp, _vp, _vp]),

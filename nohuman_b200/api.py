@@ -277,6 +277,29 @@ class Database:
                                            items_per_chain, iters, C.byref(a), C.byref(b)))
         return a.value, b.value
 
+    def taxon_counts(self):
+        """(counts, occupied, out_of_range) of the resident table, counted on its device (nh_db_taxon_counts):
+        counts[node] is the number of cells holding internal taxon id `node` (uint64, node_count entries, counts[0]
+        is 0), occupied the cells with a non-zero value, out_of_range those whose value is not a taxo.k2d node."""
+        n = int(self.info.node_count)
+        counts = np.zeros(n, np.uint64)
+        occ, oor = C.c_uint64(), C.c_uint64()
+        check(lib().nh_db_taxon_counts(self._h, counts.ctypes.data, n, C.byref(occ), C.byref(oor)))
+        return counts, int(occ.value), int(oor.value)
+
+    def inspect(self, path=None, skip_counts: bool = False, zero_counts: bool = False) -> None:
+        """What `kraken2-inspect` prints for this database (nh_db_inspect), to `path` (None: stdout).  NhError
+        NH_ERR_IO, with nothing written, when a cell's value is not a taxo.k2d node or the occupied cells differ
+        from the header's size."""
+        flags = (_ffi.NH_INSPECT_SKIP_COUNTS if skip_counts else 0) | (_ffi.NH_INSPECT_ZERO_COUNTS if zero_counts else 0)
+        check(lib().nh_db_inspect(self._h, None if path is None else str(path).encode(), flags))
+
+    def taxon_counts_kernel_seconds(self, iters: int = 10) -> float:
+        """Device time of one taxon-count pass over the table (nh_bench_taxon_counts), mean of `iters`."""
+        t = C.c_double()
+        check(lib().nh_bench_taxon_counts(self._h, int(iters), C.byref(t)))
+        return t.value
+
     def close(self) -> None:
         if self._h:
             lib().nh_db_close(self._h)

@@ -4,6 +4,7 @@
 
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <stdio.h>
 
 #include <functional>
 #include <string>
@@ -213,6 +214,12 @@ class NhSeqReader {
   struct Impl;
   Impl *impl_;
 };
+
+/* nh_pipeline.cc: kraken2's report (reports.cc ReportKrakenStyle) to f: counts[node] are the direct counts, total
+ * the count the percentages are of.  The "unclassified" line comes first when `unclassified` is non-zero or with
+ * zero_counts, which also lists every node, zero counts included (--report-zero-counts).  false: a write failed. */
+bool write_report(FILE *f, const nh_db *db, const std::vector<uint64_t> &counts, uint64_t total, uint64_t unclassified,
+                  bool zero_counts);
 
 int nh_set_error(int code, const char *fmt, ...);
 int nh_db_build_filter(nh_db *db); /* after the cells are on the device (every open path; the synthetic builder calls it itself) */

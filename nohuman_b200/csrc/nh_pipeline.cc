@@ -1214,11 +1214,11 @@ static void append_kraken_line(std::string &out, const Work &w, uint64_t i, int 
   out.push_back('\n');
 }
 
+}  // namespace
+
 /* kraken2 report (reports.cc ReportKrakenStyle): percentage, clade count, direct count, rank code, taxid, indented name */
-static bool write_report(const char *path, const nh_db *db, const std::vector<uint64_t> &call_counts, uint64_t total,
-                         uint64_t unclassified) {
-  FILE *f = fopen(path, "w");
-  if (!f) return false;
+bool write_report(FILE *f, const nh_db *db, const std::vector<uint64_t> &call_counts, uint64_t total, uint64_t unclassified,
+                  bool zero_counts) {
   const size_t n = db->h_parent.size();
   std::vector<uint64_t> clade(call_counts);
   for (size_t i = n; i-- > 2;) clade[db->h_parent[i]] += clade[i]; /* parent id < child id */
@@ -1229,7 +1229,7 @@ static bool write_report(const char *path, const nh_db *db, const std::vector<ui
             (unsigned long long)cl, (unsigned long long)direct, rank.c_str(), (unsigned long long)taxid, 2 * depth, "",
             name.c_str());
   };
-  if (unclassified) line(unclassified, unclassified, "U", 0, "unclassified", 0);
+  if (unclassified || zero_counts) line(unclassified, unclassified, "U", 0, "unclassified", 0);
   struct Frame {
     uint32_t id;
     char code;
@@ -1240,7 +1240,7 @@ static bool write_report(const char *path, const nh_db *db, const std::vector<ui
   while (!stack.empty()) {
     Frame fr = stack.back();
     stack.pop_back();
-    if (clade[fr.id] == 0) continue;
+    if (clade[fr.id] == 0 && !zero_counts) continue;
     const std::string &rank = db->h_rank[fr.id];
     static const std::pair<const char *, char> codes[] = {{"superkingdom", 'D'}, {"kingdom", 'K'}, {"phylum", 'P'}, {"class", 'C'},
                                                           {"order", 'O'},        {"family", 'F'},  {"genus", 'G'},  {"species", 'S'}};
@@ -1259,8 +1259,10 @@ static bool write_report(const char *path, const nh_db *db, const std::vector<ui
     std::stable_sort(ch.begin(), ch.end(), [&](uint32_t a, uint32_t b) { return clade[a] > clade[b]; });
     for (auto it = ch.rbegin(); it != ch.rend(); ++it) stack.push_back({*it, fr.code, fr.rank_depth, fr.depth + 1});
   }
-  return fclose(f) == 0;
+  return !ferror(f);
 }
+
+namespace {
 
 static int run_pipeline(const Decider &dec, const nh_files_t *files, nh_run_stats_t *stats) {
   const auto t0 = std::chrono::steady_clock::now();
@@ -1556,10 +1558,14 @@ static int run_pipeline(const Decider &dec, const nh_files_t *files, nh_run_stat
       fail_msg = std::string("writing ") + files->kraken_output + " failed";
     }
   }
-  if (want_report && !failed &&
-      !write_report(files->kraken_report, dec.dbs[0], call_counts, total_units, total_units - n_classified)) {
-    failed = true;
-    fail_msg = std::string("writing ") + files->kraken_report + " failed";
+  if (want_report && !failed) {
+    FILE *rf = fopen(files->kraken_report, "w");
+    bool ok = rf && write_report(rf, dec.dbs[0], call_counts, total_units, total_units - n_classified, false);
+    if (rf) ok = fclose(rf) == 0 && ok;
+    if (!ok) {
+      failed = true;
+      fail_msg = std::string("writing ") + files->kraken_report + " failed";
+    }
   }
   if (failed) return nh_set_error(NH_ERR_IO, "%s", fail_msg.c_str());
   std::string deflate_msg;

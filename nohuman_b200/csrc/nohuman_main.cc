@@ -587,6 +587,53 @@ static int dustmasker_shim(int argc, char **argv) {
   return 0;
 }
 
+/* kraken2-inspect --db DIR [--skip-counts] [--report-zero-counts]: the database's options and its minimizers per
+ * taxon, counted on the GPU (nh_db_inspect), to stdout.  --threads and --memory-mapping are accepted and do nothing
+ * (the table goes to the GPU either way); --gpu N picks the device.  Any other option is refused with one line. */
+static int kraken2_inspect_shim(int argc, char **argv) {
+  static option opts[] = {{"db", 1, 0, 'd'},           {"skip-counts", 0, 0, 's'},    {"report-zero-counts", 0, 0, 'z'},
+                          {"threads", 1, 0, 't'},      {"memory-mapping", 0, 0, 'm'}, {"gpu", 1, 0, 'g'},
+                          {"use-mpa-style", 0, 0, 1},  {0, 0, 0, 0}};
+  std::string db;
+  int flags = 0, gpu = 0, c;
+  opterr = 0; /* the refusals below are the only message */
+  while ((c = getopt_long(argc, argv, ":", opts, nullptr)) != -1) switch (c) {
+      case 'd': db = optarg; break;
+      case 's': flags |= NH_INSPECT_SKIP_COUNTS; break;
+      case 'z': flags |= NH_INSPECT_ZERO_COUNTS; break;
+      case 't': case 'm': break;
+      case 'g': gpu = atoi(optarg); break;
+      case 1:
+        fprintf(stderr, "kraken2-inspect (GPU): --use-mpa-style is not supported (kraken-style reports only)\n");
+        return 64;
+      case ':':
+        fprintf(stderr, "kraken2-inspect (GPU): option %s needs a value\n", argv[optind - 1]);
+        return 64;
+      default: {
+        const std::string o = optopt ? std::string("-") + (char)optopt : std::string(argv[optind - 1]);
+        fprintf(stderr, "kraken2-inspect (GPU): option %s is not supported (--db, --skip-counts, --report-zero-counts, "
+                        "--threads, --memory-mapping, --gpu)\n", o.c_str());
+        return 64;
+      }
+    }
+  if (optind < argc) {
+    fprintf(stderr, "kraken2-inspect (GPU): unexpected argument %s\n", argv[optind]);
+    return 64;
+  }
+  if (db.empty()) {
+    fprintf(stderr, "kraken2-inspect (GPU): --db DIR is required\n");
+    return 64;
+  }
+  nh_db *dbh = nullptr;
+  if (nh_db_open(db.c_str(), gpu, &dbh) || nh_db_inspect(dbh, nullptr, flags)) {
+    const int rc = fail("kraken2-inspect: %s", nh_last_error());
+    nh_db_close(dbh);
+    return rc;
+  }
+  nh_db_close(dbh);
+  return 0;
+}
+
 /* ------------------------------------------------------------------ */
 
 static void usage() {
@@ -617,6 +664,7 @@ int main(int argc, char **argv) {
   if (path_file_name(argv[0]) == "kraken2") return kraken2_shim(argc, argv);
   if (path_file_name(argv[0]) == "kraken2-build") return kraken2_build_shim(argc, argv);
   if (path_file_name(argv[0]) == "dustmasker") return dustmasker_shim(argc, argv);
+  if (path_file_name(argv[0]) == "kraken2-inspect") return kraken2_inspect_shim(argc, argv);
   static option opts[] = {{"out1", 1, 0, 'o'},         {"out2", 1, 0, 'O'},          {"check", 0, 0, 'c'},
                           {"download", 0, 0, 'd'},     {"db", 1, 0, 'D'},            {"db-version", 1, 0, 1},
                           {"list-db-versions", 0, 0, 2}, {"output-type", 1, 0, 'F'}, {"threads", 1, 0, 't'},
